@@ -17,9 +17,14 @@ __version__ = "0.1.0"
 _LAZY = {"TradingVectorEnv", "MultiDatasetTradingVectorEnv", "basic_reward_function",
          "dynamic_feature_last_position_taken", "dynamic_feature_real_position", "shard_envs", "LazyInfos",
          "DeviceReward", "log_return_reward", "simple_return_reward"}
+_FEATURES = {"DeviceFeature", "parse_dynamic_features", "portfolio_return_feature", "reward_feature",
+             "episode_progress_feature"}
 
 
 def __getattr__(name):          # torch / the CUDA library are only imported when an env class is used
+    if name in _FEATURES:             # host-only: importable without torch or a device
+        from . import dynamic_features
+        return getattr(dynamic_features, name)
     if name in _LAZY:
         from . import vector_env
         return getattr(vector_env, name)

@@ -24,6 +24,15 @@ GTE_MAX_DATASETS = 64
 GTE_N_METRICS = 8
 GTE_STEP_THREADS = 256
 GTE_MAX_PARTIAL_ROWS = 4096
+GTE_MAX_DYN = 5
+
+
+def ring_tile_bytes(windows: int, n_dyn: int, dyn_kinds: int) -> int:
+    """Bytes of one 32-env tile of the dynamic-feature ring (GTE_RING_TILE_BYTES_DYN): W rows x 32 f32 values per f32
+    kind, plus W rows x 32 u8 position indices when "position" (kind 1) is a column; dyn_kinds 0 = the default pair."""
+    W = max(int(windows), 1)
+    n_pos = sum(((dyn_kinds >> (4 * j)) & 15) == 1 for j in range(n_dyn)) if dyn_kinds else 1
+    return W * (128 * (n_dyn - n_pos) + 32 * n_pos)
 REWARD_LOG_RETURN, REWARD_SIMPLE_RETURN = 0, 1
 OBS_AUTO, OBS_GENERIC, OBS_VEC, OBS_TMA = 0, 1, 2, 3
 OBS_VARIANTS = {"auto": OBS_AUTO, "generic": OBS_GENERIC, "vec": OBS_VEC, "tma": OBS_TMA}
@@ -39,7 +48,7 @@ class GteParams(C.Structure):
         ("episodes_between_switch", C.c_int32), ("plan_episodes", C.c_int32),
         ("multi_dataset", C.c_int32), ("reward_kind", C.c_int32),
         ("n_limit_positions", C.c_int32), ("action_bytes", C.c_int32),
-        ("strict_actions", C.c_int32), ("reserved0", C.c_int32),
+        ("strict_actions", C.c_int32), ("dyn_kinds", C.c_int32),
         ("t_stride", C.c_int64), ("env_id_offset", C.c_int64), ("seed", C.c_uint64),
         ("fee", C.c_double), ("rate", C.c_double), ("v0", C.c_double), ("done_ratio", C.c_double),
         ("reward_scale", C.c_double), ("reward_lo", C.c_double), ("reward_hi", C.c_double),

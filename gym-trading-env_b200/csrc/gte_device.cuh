@@ -160,6 +160,65 @@ __device__ __forceinline__ void ring_store(const GteParams& P, const GteState& S
     tile[GTE_RING_POS_OFFSET(W, slot, e)] = (uint8_t)pos_idx;
 }
 
+// Dynamic-column descriptor, derived once on the host from (n_dyn, dyn_kinds) by dyn_layout(): drives the ring layout
+// (include/gte_b200.h, GteState.dyn_ring) on both the step and the gather side.  `general` is false for no dynamic
+// columns and for the default pair (position, real_position): those run the kernels' original instantiations.
+constexpr uint32_t kDynPosBlock = 0xF, kDynNone = 0xE;
+struct DynLayout {
+    uint32_t col_src;     // nibble j: the ring block column j reads: f32 block 0..3, or kDynPosBlock (u8 position indices)
+    uint32_t kind_blk;    // nibble k (enum GteDynKind): the block of kind k, or kDynNone when it is not configured
+    int n_f32, n_pos;     // f32 blocks, position-index blocks (0 or 1)
+    int tile_bytes;       // GTE_RING_TILE_BYTES_DYN(W, n_f32, n_pos)
+    bool general;
+};
+
+// dyn_kinds with the legacy 0 spelled out (n_dyn == 2: the default pair, 0x21)
+static inline uint32_t dyn_kinds_of(const GteParams& P) {
+    return (P.dyn_kinds == 0 && P.n_dyn == 2) ? 0x21u : (uint32_t)P.dyn_kinds;
+}
+
+static inline DynLayout dyn_layout(const GteParams& P) {
+    DynLayout L;
+    const uint32_t kinds = dyn_kinds_of(P);
+    const int W = P.windows > 0 ? P.windows : 1;
+    L.n_pos = 0;
+    for (int j = 0; j < P.n_dyn; ++j) L.n_pos += ((kinds >> (4 * j)) & 15u) == GTE_DYN_POSITION;
+    L.n_f32 = P.n_dyn - L.n_pos;
+    L.kind_blk = 0u;
+    for (int k = 0; k < 8; ++k) L.kind_blk |= kDynNone << (4 * k);
+    int blk = 0;
+    for (int k = GTE_DYN_REAL_POSITION; k <= GTE_DYN_EPISODE_PROGRESS; ++k)     // f32 blocks in kind-code order
+        for (int j = 0; j < P.n_dyn; ++j)
+            if (((kinds >> (4 * j)) & 15u) == (uint32_t)k) L.kind_blk = (L.kind_blk & ~(15u << (4 * k))) | ((uint32_t)blk++ << (4 * k));
+    if (L.n_pos) L.kind_blk = (L.kind_blk & ~(15u << (4 * GTE_DYN_POSITION))) | (kDynPosBlock << (4 * GTE_DYN_POSITION));
+    L.col_src = 0u;
+    for (int j = 0; j < P.n_dyn; ++j) L.col_src |= ((L.kind_blk >> (4 * ((kinds >> (4 * j)) & 15u))) & 15u) << (4 * j);
+    L.tile_bytes = GTE_RING_TILE_BYTES_DYN(W, L.n_f32, L.n_pos);
+    L.general = P.n_dyn > 0 && kinds != 0x21u;
+    return L;
+}
+
+__device__ __forceinline__ uint32_t dyn_block_of(const DynLayout& L, int kind) { return (L.kind_blk >> (4 * kind)) & 15u; }
+
+// One row of every configured dynamic column (general catalogue), fp64 values already cast to f32 as numpy casts (:154).
+struct DynRow {
+    float rp, pr, rew, prog;      // real_position, portfolio_return, reward, episode_progress
+    int pos_idx;                  // position: index into positions
+};
+__device__ __forceinline__ void ring_store_dyn(const GteParams& P, const DynLayout& L, const GteState& S, int i, int slot,
+                                               const DynRow& r) {
+    const int W = P.windows > 0 ? P.windows : 1;
+    const int e = i & 31;
+    uint8_t* tile = S.dyn_ring + (int64_t)(i >> 5) * L.tile_bytes;
+    const float v[4] = {r.rp, r.pr, r.rew, r.prog};
+#pragma unroll
+    for (int k = GTE_DYN_REAL_POSITION; k <= GTE_DYN_EPISODE_PROGRESS; ++k) {
+        const uint32_t b = dyn_block_of(L, k);
+        if (b < kDynNone) *reinterpret_cast<float*>(tile + GTE_RING_F32_OFFSET(W, (int)b, slot, e)) = v[k - GTE_DYN_REAL_POSITION];
+    }
+    if (L.n_pos) tile[GTE_RING_POS_OFFSET_DYN(W, L.n_f32, slot, e)] = (uint8_t)r.pos_idx;
+}
+
 struct EnvRegs {          // the per-env state a step keeps in registers
     Portfolio pf;
     int pos_idx, step, ep_start, ds;
@@ -167,8 +226,10 @@ struct EnvRegs {          // the per-env state a step keeps in registers
 
 // TradingEnv.reset (environments.py:163-199) preceded by MultiDatasetTradingEnv.reset (:393-400).
 // Rare path (once per episode): plan/rotation bookkeeping goes straight to global memory.
+// GEN: the general dynamic-feature catalogue (L.general), else no dynamic columns or the default pair.
+template <bool GEN = false>
 __device__ __forceinline__ void reset_env(const GteParams& P, const GteData& D, const GteState& S,
-                                       int i, uint64_t tick, int ring_slot, EnvRegs& e) {
+                                       int i, uint64_t tick, int ring_slot, EnvRegs& e, const DynLayout& L) {
     uint32_t r[4];
     philox_draw(P.seed, tick, (uint64_t)(P.env_id_offset + i), r);
     const bool have_plan = P.plan_episodes > 0 && S.reset_plan != nullptr;
@@ -217,8 +278,12 @@ __device__ __forceinline__ void reset_env(const GteParams& P, const GteData& D, 
     e.pf = target_portfolio(position, P.v0, price);                          // :179-183
     for (int k = 0; k < P.n_limit_positions; ++k)                            // self._limit_orders = {} (:168)
         S.limit_price[(int64_t)i * P.n_positions + S.limit_seq[k]] = __longlong_as_double(0x7ff8000000000000ll);
-    if (P.n_dyn > 0)                                                         // first obs row: (position, position) :191-192
+    if (GEN) {                                // first obs row (:191-192): position, real_position = position, else 0
+        const DynRow r = {(float)position, 0.0f, 0.0f, 0.0f, e.pos_idx};
+        ring_store_dyn(P, L, S, i, ring_slot, r);
+    } else if (P.n_dyn > 0) {                                                // first obs row: (position, position) :191-192
         ring_store(P, S, i, ring_slot, (float)position, e.pos_idx);
+    }
 }
 
 }  // namespace gte

@@ -18,8 +18,25 @@
 
 namespace gte {
 
+// One dynamic column of the general catalogue (GEN instantiations): column j of env lane e in ring slot s of a tile
+// (CG: a global-memory tile read through L2 only, as the vec gather reads the ring).
+template <bool CG = false>
+__device__ __forceinline__ float dyn_ring_value(const GteParams& P, const ObsShape& sh, const uint8_t* tile, int j, int s, int e) {
+    const uint32_t src = (sh.dyn.col_src >> (4 * j)) & 15u;
+    if (src == kDynPosBlock) {
+        const uint8_t* p = tile + GTE_RING_POS_OFFSET_DYN(sh.W, sh.dyn.n_f32, s, e);
+        return (float)P.positions[CG ? __ldcg(p) : *p];
+    }
+    const float* p = reinterpret_cast<const float*>(tile + GTE_RING_F32_OFFSET(sh.W, (int)src, s, e));
+    return CG ? __ldcg(p) : *p;
+}
+__device__ __forceinline__ const uint8_t* ring_tile_dyn(const GteState& S, const ObsShape& sh, int64_t env) {
+    return S.dyn_ring + (env >> 5) * (int64_t)sh.dyn.tile_bytes;
+}
+
 // ------------------------------------------------------------------------------------------ generic
-template <int G>
+// GEN (every kernel below): dynamic columns of the general catalogue (sh.dyn), else none or the default pair.
+template <int G, bool GEN = false>
 __global__ void __launch_bounds__(256)
 obs_generic_kernel(const GteParams P, const GteData D, const GteState S, float* __restrict__ obs,
                    const ObsShape sh, const int env_begin, const int env_end) {
@@ -45,11 +62,15 @@ obs_generic_kernel(const GteParams P, const GteData D, const GteState S, float* 
                 const int r = r0 + w;
                 int slot = s0 + w;
                 if (slot >= sh.W) slot -= sh.W;
-                const uint8_t* __restrict__ ring = ring_tile(S, sh.W, env);
                 const int e32 = (int)(env & 31);
-                v = (r < ep_start) ? 0.0f
-                  : (c == sh.ns ? (float)P.positions[ring[GTE_RING_POS_OFFSET(sh.W, slot, e32)]]
-                                : *reinterpret_cast<const float*>(ring + GTE_RING_RP_OFFSET(slot, e32)));
+                if (GEN) {
+                    v = (r < ep_start) ? 0.0f : dyn_ring_value(P, sh, ring_tile_dyn(S, sh, env), c - sh.ns, slot, e32);
+                } else {
+                    const uint8_t* __restrict__ ring = ring_tile(S, sh.W, env);
+                    v = (r < ep_start) ? 0.0f
+                      : (c == sh.ns ? (float)P.positions[ring[GTE_RING_POS_OFFSET(sh.W, slot, e32)]]
+                                    : *reinterpret_cast<const float*>(ring + GTE_RING_RP_OFFSET(slot, e32)));
+                }
             }
             out[e] = v;
         }
@@ -69,7 +90,7 @@ __device__ __forceinline__ void st_cs_v4(void* p, const float4& v) {
 }
 
 // ------------------------------------------------------------------------------------------ vec
-template <bool PAIR>     // PAIR: n_dyn == 2 and F even -> the dynamic pair is an aligned float2
+template <bool PAIR, bool GEN = false>     // PAIR: the default pair and F even -> the dynamic pair is an aligned float2
 __global__ void __launch_bounds__(256)
 obs_vec_kernel(const GteParams P, const GteData D, const GteState S, float* __restrict__ obs,
                const ObsShape sh, const int env_begin, const int env_end) {
@@ -83,7 +104,7 @@ obs_vec_kernel(const GteParams P, const GteData D, const GteState S, float* __re
         const int ds = S.dataset_idx[env];
         const int r0 = idx + 1 - sh.W;
         const char* __restrict__ src = window_src(D, sh, ds, r0);
-        const uint8_t* __restrict__ ring = ring_tile(S, sh.W, env);
+        const uint8_t* __restrict__ ring = GEN ? ring_tile_dyn(S, sh, env) : ring_tile(S, sh.W, env);
         const int e32 = (int)(env & 31);
         char* __restrict__ dst = reinterpret_cast<char*>(obs) + env * (int64_t)sh.win_bytes;
         for (int j = lane; j < sh.n_vec; j += 32) {
@@ -99,6 +120,10 @@ obs_vec_kernel(const GteParams P, const GteData D, const GteState S, float* __re
                         const int r = r0 + w;
                         int slot = s0 + w;
                         if (slot >= sh.W) slot -= sh.W;
+                        if (GEN) {
+                            pv[k] = (r < ep_start) ? 0.0f : dyn_ring_value<true>(P, sh, ring, c - sh.ns, slot, e32);
+                            continue;
+                        }
                         const uint8_t* rpos = ring + GTE_RING_POS_OFFSET(sh.W, slot, e32);
                         const float* rrp = reinterpret_cast<const float*>(ring + GTE_RING_RP_OFFSET(slot, e32));
                         if (PAIR) {
@@ -125,9 +150,9 @@ obs_vec_kernel(const GteParams P, const GteData D, const GteState S, float* __re
 //                   waits for a free window stage (empty mbarrier), publishes the first live rows to shared
 //                   memory and issues the group's G cp.async.bulk window copies from the L2-resident window
 //                   table onto the stage's full mbarrier.  One tile ahead it issues the ONE cp.async.bulk of the
-//                   tile's dynamic-feature ring block (HBM, W x 160 contiguous bytes: real_position rows whose
-//                   16-byte chunks are XOR-swizzled so the consumers' column reads spread over the banks, then
-//                   position-index rows);
+//                   tile's dynamic-feature ring block (HBM, contiguous: W x 160 bytes for the default pair — real_position
+//                   rows whose 16-byte chunks are XOR-swizzled so the consumers' column reads spread over the banks,
+//                   then position-index rows; GTE_RING_TILE_BYTES_DYN for the general catalogue);
 //   consumer warps: wait on both full mbarriers, patch the dynamic columns smem->smem (128 threads = G envs x
 //                   128/G slots per pass; rows before the episode start stay zero), fence.proxy.async, and each
 //                   warp arrives on the stage's ready mbarrier (and, after the tile's last group, hands the ring
@@ -169,7 +194,7 @@ struct FusedStep {
 // same stream handed out on demand 7.4-7.6 TB/s — the SMs do not all reach memory equally fast, and with a static split
 // the launch lasts as long as the slowest of them.  The producer publishes each tile id through shared memory (ring of 4
 // ids, riding on the release of the stage's full barrier); a tile id past the end stops consumers and store warp.
-template <int WS, int RT, int G, int UNIT = kTileEnvs, bool FUSED = false, bool DYN = false>
+template <int WS, int RT, int G, int UNIT = kTileEnvs, bool FUSED = false, bool DYN = false, bool GEN = false>
 __global__ void __launch_bounds__(kCoopThreads, FUSED ? 4 : 1)
 obs_tma_coop_kernel(const GteParams P, const GteData D, const GteState S, float* __restrict__ obs,
                     const ObsShape sh, const int env_begin, const int env_end, const FusedStep FS) {
@@ -196,7 +221,9 @@ obs_tma_coop_kernel(const GteParams P, const GteData D, const GteState S, float*
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const bool ring = sh.nd > 0;
     const uint32_t win_bytes = (uint32_t)sh.win_bytes;
-    const uint32_t wstage_bytes = win_bytes * G, rstride = (uint32_t)GTE_RING_TILE_BYTES(sh.W);
+    const uint32_t wstage_bytes = win_bytes * G;
+    const uint32_t rstride = GEN ? (uint32_t)sh.dyn.tile_bytes : (uint32_t)GTE_RING_TILE_BYTES(sh.W);
+    auto ring_src = [&](int64_t env) -> const uint8_t* { return GEN ? ring_tile_dyn(S, sh, env) : ring_tile(S, sh.W, env); };
     unsigned char* rbase = smem_raw;
     unsigned char* wbase = rbase + (ring ? (size_t)RT * rstride : 0);
 
@@ -230,7 +257,7 @@ obs_tma_coop_kernel(const GteParams P, const GteData D, const GteState S, float*
         for (int j = tid; j < kFusedMaxEnvs; j += kCoopThreads) {          // (the launcher guarantees the CTA owns <= 256 envs)
             const int64_t env = tile_env0(j / unit_envs) + (j % unit_envs);
             if (env < env_end) {
-                const StepThreadOut r = step_env_now(P, D, S, FS.actions, K, FS.O, tick, ring_slot, FS.autoreset, (int)env, acc, f_pos);
+                const StepThreadOut r = step_env_now<GEN>(P, D, S, FS.actions, K, FS.O, tick, ring_slot, FS.autoreset, (int)env, acc, f_pos);
                 f_live[j] = sh.W - 1 - (r.idx - r.ep_start);             // window row of ep_start (<= 0: the whole window is live)
                 f_src[j] = (unsigned long long)window_src(D, sh, r.ds, r.idx + 1 - sh.W);
             }
@@ -273,7 +300,7 @@ obs_tma_coop_kernel(const GteParams P, const GteData D, const GteState S, float*
                 const int stage = k % RT, use = k / RT;
                 if (use > 0) mbar_wait(&empty_r[stage], (uint32_t)(use - 1) & 1u);
                 mbar_expect_tx(&full_r[stage], rstride);
-                bulk_g2s(rbase + (size_t)stage * rstride, ring_tile(S, sh.W, tile_env0(k)), rstride, &full_r[stage]);
+                bulk_g2s(rbase + (size_t)stage * rstride, ring_src(tile_env0(k)), rstride, &full_r[stage]);
             }
         };
         if (DYN) {
@@ -293,7 +320,7 @@ obs_tma_coop_kernel(const GteParams P, const GteData D, const GteState S, float*
                     const int stage = k % RT, use = k / RT;
                     if (use > 0) mbar_wait(&empty_r[stage], (uint32_t)(use - 1) & 1u);
                     mbar_expect_tx(&full_r[stage], rstride);
-                    bulk_g2s(rbase + (size_t)stage * rstride, ring_tile(S, sh.W, env0_of(t)), rstride, &full_r[stage]);
+                    bulk_g2s(rbase + (size_t)stage * rstride, ring_src(env0_of(t)), rstride, &full_r[stage]);
                 }
             };
             // lane 0 claims; the answer of a claim is only looked at one whole tile later (claim_use), so the round trip of
@@ -445,8 +472,12 @@ obs_tma_coop_kernel(const GteParams P, const GteData D, const GteState S, float*
                             if (w < 0) w += sh.W;
                             if (w >= live0) {                    // rows before the episode start stay zero
                                 float* qd = fbuf + w * sh.F + sh.ns;
-                                qd[0] = (float)P.positions[rtile[GTE_RING_POS_OFFSET(sh.W, s, e)]];   // fp64 -> fp32 as numpy casts (:154)
-                                qd[1] = *reinterpret_cast<const float*>(rtile + GTE_RING_RP_OFFSET(s, e));
+                                if (GEN) {
+                                    for (int j = 0; j < sh.nd; ++j) qd[j] = dyn_ring_value(P, sh, rtile, j, s, e);
+                                } else {
+                                    qd[0] = (float)P.positions[rtile[GTE_RING_POS_OFFSET(sh.W, s, e)]];   // fp64 -> fp32 as numpy casts (:154)
+                                    qd[1] = *reinterpret_cast<const float*>(rtile + GTE_RING_RP_OFFSET(s, e));
+                                }
                             }
                         }
                     }
@@ -480,14 +511,50 @@ using ObsKernelFn = void (*)(const GteParams, const GteData, const GteState, flo
 struct TmaConfig { int wstages, rtiles, group; };
 
 static size_t tma_smem_bytes(const ObsShape& sh, const TmaConfig& c) {
-    const size_t ring = sh.nd > 0 ? (size_t)c.rtiles * GTE_RING_TILE_BYTES(sh.W) : 0;
+    const size_t ring = sh.nd > 0 ? (size_t)c.rtiles * sh.dyn.tile_bytes : 0;
     return (size_t)c.group * c.wstages * sh.win_bytes + ring;
 }
 
-static ObsKernelFn tma_kernel(const TmaConfig& c, int unit = kTileEnvs, bool fused = false, bool dyn = false) {
+// The general dynamic-feature catalogue: the default pipeline shape (3 window stages, 2 ring tiles, the group sizes
+// tma_config() may pick) in every form.
+static ObsKernelFn tma_kernel_gen(int key, int unit, bool fused, bool dyn) {
+    if (dyn) {
+        if (fused || unit != kTileEnvs) return nullptr;
+        switch (key) {
+            case 30201: return obs_tma_coop_kernel<3, 2, 1, 32, false, true, true>;
+            case 30202: return obs_tma_coop_kernel<3, 2, 2, 32, false, true, true>;
+            case 30204: return obs_tma_coop_kernel<3, 2, 4, 32, false, true, true>;
+            default: return nullptr;
+        }
+    }
+    switch ((fused ? 1000000 : 0) + unit * 100000 + key) {
+        case 3230201: return obs_tma_coop_kernel<3, 2, 1, 32, false, false, true>;
+        case 3230202: return obs_tma_coop_kernel<3, 2, 2, 32, false, false, true>;
+        case 3230204: return obs_tma_coop_kernel<3, 2, 4, 32, false, false, true>;
+        case 1630201: return obs_tma_coop_kernel<3, 2, 1, 16, false, false, true>;
+        case 1630202: return obs_tma_coop_kernel<3, 2, 2, 16, false, false, true>;
+        case 1630204: return obs_tma_coop_kernel<3, 2, 4, 16, false, false, true>;
+        case 830201: return obs_tma_coop_kernel<3, 2, 1, 8, false, false, true>;
+        case 830202: return obs_tma_coop_kernel<3, 2, 2, 8, false, false, true>;
+        case 830204: return obs_tma_coop_kernel<3, 2, 4, 8, false, false, true>;
+        case 4230201: return obs_tma_coop_kernel<3, 2, 1, 32, true, false, true>;
+        case 4230202: return obs_tma_coop_kernel<3, 2, 2, 32, true, false, true>;
+        case 4230204: return obs_tma_coop_kernel<3, 2, 4, 32, true, false, true>;
+        case 2630201: return obs_tma_coop_kernel<3, 2, 1, 16, true, false, true>;
+        case 2630202: return obs_tma_coop_kernel<3, 2, 2, 16, true, false, true>;
+        case 2630204: return obs_tma_coop_kernel<3, 2, 4, 16, true, false, true>;
+        case 1830201: return obs_tma_coop_kernel<3, 2, 1, 8, true, false, true>;
+        case 1830202: return obs_tma_coop_kernel<3, 2, 2, 8, true, false, true>;
+        case 1830204: return obs_tma_coop_kernel<3, 2, 4, 8, true, false, true>;
+        default: return nullptr;
+    }
+}
+
+static ObsKernelFn tma_kernel(const TmaConfig& c, int unit = kTileEnvs, bool fused = false, bool dyn = false, bool gen = false) {
     // (window stages, ring-tile stages, envs per group) combinations compiled in; smaller work units, the fused
     // step+gather form and the claimed-tiles form (large batches) for the default shapes
     const int key = c.wstages * 10000 + c.rtiles * 100 + c.group;
+    if (gen) return tma_kernel_gen(key, unit, fused, dyn);
     if (dyn) {
         if (fused || unit != kTileEnvs) return nullptr;
         switch (key) {
@@ -553,9 +620,21 @@ static TmaConfig tma_config(const ObsShape& sh) {
     static const int g = [] { const char* e = getenv("GTE_TMA_GROUP"); return e ? atoi(e) : 0; }();
     if (ws > 0 && rt > 0 && g > 0) {
         const TmaConfig c{ws, rt, g};
-        if (tma_kernel(c) != nullptr) return c;
+        if (tma_kernel(c, kTileEnvs, false, false, sh.dyn.general) != nullptr) return c;
     }
     TmaConfig c{3, 2, 4};
+    if (sh.dyn.general) {
+        // the general catalogue's ring stages grow with its f32 columns (W x 544 bytes per tile with all five): halving
+        // the group no longer buys a CTA per SM, so take the group with the most windows in flight per SM
+        int best = 0;
+        for (int g = 4; g >= 1; g /= 2) {
+            const TmaConfig t{3, 2, g};
+            const size_t smem = tma_smem_bytes(sh, t);
+            const int in_flight = (int)((227u * 1024u) / (smem + 2048u)) * g;
+            if (smem <= 200 * 1024 && in_flight > best) { best = in_flight; c = t; }
+        }
+        return c;
+    }
     while (c.group > 1 && tma_smem_bytes(sh, c) > 100 * 1024) c.group /= 2;
     return c;
 }
@@ -575,7 +654,7 @@ bool obs_vec_supported(const GteParams& P, const GteData& D) {
 bool obs_tma_supported(const GteParams& P, const GteData& D) {
     if (!obs_vec_supported(P, D)) return false;
     const ObsShape sh = make_shape(P);
-    return (sh.nd == 0 || sh.nd == 2) && tma_smem_bytes(sh, tma_config(sh)) <= 200 * 1024;
+    return tma_smem_bytes(sh, tma_config(sh)) <= 200 * 1024;
 }
 
 // Grid / work-unit choice of the TMA gather for n_envs envs (and the one-time per-device kernel attribute opt-ins).
@@ -608,7 +687,8 @@ static unsigned int* dyn_sched_slot(cudaStream_t stream) {
 static cudaError_t plan_tma(const ObsShape& sh, int n_envs, bool fused, TmaPlan* out, cudaStream_t stream = nullptr) {
     const TmaConfig cfg = tma_config(sh);
     const size_t smem = tma_smem_bytes(sh, cfg);
-    ObsKernelFn probe = tma_kernel(cfg, kTileEnvs, fused);
+    const bool gen = sh.dyn.general;
+    ObsKernelFn probe = tma_kernel(cfg, kTileEnvs, fused, false, gen);
     if (probe == nullptr) return cudaErrorInvalidValue;
     int dev = 0;
     cudaGetDevice(&dev);
@@ -647,8 +727,8 @@ static cudaError_t plan_tma(const ObsShape& sh, int n_envs, bool fused, TmaPlan*
     int64_t best = -1;
     static const int forced_unit = [] { const char* e = getenv("GTE_TMA_UNIT"); return e ? atoi(e) : 0; }();   // tuning runs
     for (int u = 32; u >= 8 && u >= cfg.group; u /= 2) {
-        if (forced_unit > 0 && tma_kernel(cfg, forced_unit, fused) != nullptr) { unit = forced_unit; break; }
-        if (tma_kernel(cfg, u, fused) == nullptr) continue;
+        if (forced_unit > 0 && tma_kernel(cfg, forced_unit, fused, false, gen) != nullptr) { unit = forced_unit; break; }
+        if (tma_kernel(cfg, u, fused, false, gen) == nullptr) continue;
         const int64_t units = ((int64_t)n_envs + u - 1) / u;
         const int64_t per_cta = (units + cap - 1) / cap;
         if (u == 8 && per_cta > 1) break;                  // quarter tiles only while every CTA gets at most one
@@ -665,12 +745,12 @@ static cudaError_t plan_tma(const ObsShape& sh, int n_envs, bool fused, TmaPlan*
     out->unit = unit;
     out->envs_per_cta = (int)(((need + out->grid - 1) / out->grid) * unit);
     out->smem = smem;
-    out->kern = tma_kernel(cfg, unit, fused);
+    out->kern = tma_kernel(cfg, unit, fused, false, gen);
     out->sched = nullptr;
     // large batches: tiles are claimed from a counter instead of being split evenly over the CTAs (GTE_TMA_DYN=0: never,
     // 2: whenever the kernel exists, for tests of the small-batch corners)
     static const int dyn_mode = [] { const char* e = getenv("GTE_TMA_DYN"); return e ? atoi(e) : 1; }();
-    ObsKernelFn dk = tma_kernel(cfg, unit, fused, true);
+    ObsKernelFn dk = tma_kernel(cfg, unit, fused, true, gen);
     if (dyn_mode > 0 && dk != nullptr && tiles_per_cta <= 0 &&
         (dyn_mode >= 2 || (need + out->grid - 1) / out->grid >= kDynMinTilesPerCta)) {
         unsigned int* slot = dyn_sched_slot(stream);
@@ -688,7 +768,7 @@ static cudaError_t fused_plan(const GteParams& P, const GteData& D, int variant,
     if (!enabled || P.windows <= 0 || (variant != GTE_OBS_AUTO && variant != GTE_OBS_TMA) || !obs_tma_supported(P, D))
         return cudaSuccess;
     const ObsShape sh = make_shape(P);
-    if (tma_kernel(tma_config(sh), kTileEnvs, true) == nullptr) return cudaSuccess;
+    if (tma_kernel(tma_config(sh), kTileEnvs, true, false, sh.dyn.general) == nullptr) return cudaSuccess;
     // cheap pre-check before touching kernel attributes: even 8 CTAs per SM could not keep every CTA under the limit
     if ((int64_t)P.n_envs > (int64_t)num_sms() * 8 * kFusedMaxEnvs) return cudaSuccess;
     cudaError_t e = plan_tma(sh, P.n_envs, true, plan);
@@ -732,6 +812,17 @@ cudaError_t launch_obs_range(const GteParams& P, const GteData& D, const GteStat
         while (G > 1 && G / 2 >= per_env) G /= 2;
         const int64_t need = ((int64_t)n_envs * G + 255) / 256;
         const int grid = (int)(need < (int64_t)sms * 16 ? need : (int64_t)sms * 16);
+        if (sh.dyn.general) {
+            switch (G) {
+                case 32: obs_generic_kernel<32, true><<<grid, 256, 0, stream>>>(P, D, S, obs, sh, env_begin, env_end); break;
+                case 16: obs_generic_kernel<16, true><<<grid, 256, 0, stream>>>(P, D, S, obs, sh, env_begin, env_end); break;
+                case 8: obs_generic_kernel<8, true><<<grid, 256, 0, stream>>>(P, D, S, obs, sh, env_begin, env_end); break;
+                case 4: obs_generic_kernel<4, true><<<grid, 256, 0, stream>>>(P, D, S, obs, sh, env_begin, env_end); break;
+                case 2: obs_generic_kernel<2, true><<<grid, 256, 0, stream>>>(P, D, S, obs, sh, env_begin, env_end); break;
+                default: obs_generic_kernel<1, true><<<grid, 256, 0, stream>>>(P, D, S, obs, sh, env_begin, env_end); break;
+            }
+            return cudaGetLastError();
+        }
         switch (G) {
             case 32: obs_generic_kernel<32><<<grid, 256, 0, stream>>>(P, D, S, obs, sh, env_begin, env_end); break;
             case 16: obs_generic_kernel<16><<<grid, 256, 0, stream>>>(P, D, S, obs, sh, env_begin, env_end); break;
@@ -746,7 +837,8 @@ cudaError_t launch_obs_range(const GteParams& P, const GteData& D, const GteStat
         if (!obs_vec_supported(P, D)) return cudaErrorInvalidValue;
         const int64_t need = ((int64_t)n_envs + 7) / 8;
         const int grid = (int)(need < (int64_t)sms * 8 ? need : (int64_t)sms * 8);
-        if (sh.nd == 2 && sh.F % 2 == 0) obs_vec_kernel<true><<<grid, 256, 0, stream>>>(P, D, S, obs, sh, env_begin, env_end);
+        if (sh.dyn.general) obs_vec_kernel<false, true><<<grid, 256, 0, stream>>>(P, D, S, obs, sh, env_begin, env_end);
+        else if (sh.nd == 2 && sh.F % 2 == 0) obs_vec_kernel<true><<<grid, 256, 0, stream>>>(P, D, S, obs, sh, env_begin, env_end);
         else obs_vec_kernel<false><<<grid, 256, 0, stream>>>(P, D, S, obs, sh, env_begin, env_end);
         return cudaGetLastError();
     }

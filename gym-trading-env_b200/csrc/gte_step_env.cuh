@@ -11,6 +11,7 @@ constexpr int kChunkFirst = 1, kChunkLast = 2, kChunkTotalOnly = 4;
 struct StepThreadOut {       // what the gather phase of the fused kernel needs from the step phase
     int idx, ep_start, ds;   // post-reset row index, episode start, dataset
     float dyn_pos, dyn_rp;   // the dynamic features of row idx (position, real_position), as written to the ring
+    float dyn_pr, dyn_rew, dyn_prog;   // general catalogue only: portfolio_return, reward, episode_progress of row idx
 };
 
 struct MetricAcc {           // per-thread accumulators (deterministic: fixed tile order per thread)
@@ -36,6 +37,7 @@ struct StepConsts {
                           // `valuation <= done_thr` is then bit-for-bit `valuation / v0 <= done_ratio` (:246) without the divide
     int action_bytes;     // 1, 2, 4 or 8
     int T0;               // len(df) of dataset 0, filled in ON THE DEVICE by the kernel prologue (lengths is device memory)
+    DynLayout dyn;        // dynamic-column descriptor (read by the general-catalogue instantiations only)
 };
 
 __device__ __forceinline__ void store_env(const GteState& S, int64_t i, const EnvRegs& e) {
@@ -110,8 +112,8 @@ __device__ __forceinline__ void load_prices(const GteParams& P, const GteData& D
 }
 
 // The arithmetic of one transition.  STORE_STATE = false: the caller keeps the env's state in registers across iterations
-// (rollout / server kernels) and takes it back through e_out.
-template <bool STORE_STATE = true>
+// (rollout / server kernels) and takes it back through e_out.  GEN: the general dynamic-feature catalogue (K.dyn).
+template <bool STORE_STATE = true, bool GEN = false>
 __device__ __forceinline__ StepThreadOut step_env(const GteParams& P, const GteData& D, const GteState& S,
                                                   const StepConsts& K, const GteStepOut& O, uint64_t tick, int ring_slot,
                                                   int autoreset, int i, const EnvIn& in, const double p0, const double p1,
@@ -186,8 +188,19 @@ __device__ __forceinline__ StepThreadOut step_env(const GteParams& P, const GteD
         O.pre_reset_portfolio[3 * N + i] = e.pf.ifi;
     }
     float dyn_pos = (float)pos_tab[e.pos_idx], dyn_rp = (float)rp;        // fp64 -> fp32 as numpy casts (:154)
+    float dyn_pr = 0.0f, dyn_rew = 0.0f, dyn_prog = 0.0f;
     // _get_obs write-back (:153-154); an auto-reset below overwrites the same slot with the new episode's first row
-    if (P.n_dyn > 0) ring_store(P, S, i, ring_slot, dyn_rp, e.pos_idx);
+    if (GEN) {
+        // each value only when its kind is configured (the transition is issue-bound on fp64 divides)
+        if (dyn_block_of(K.dyn, GTE_DYN_PORTFOLIO_RETURN) != kDynNone) dyn_pr = (float)dsub(ddiv(val, P.v0), 1.0);
+        dyn_rew = (float)rew;
+        if (dyn_block_of(K.dyn, GTE_DYN_EPISODE_PROGRESS) != kDynNone)
+            dyn_prog = (float)ddiv((double)e.step, (double)P.max_episode_duration);
+        const DynRow row = {dyn_rp, dyn_pr, dyn_rew, dyn_prog, e.pos_idx};
+        ring_store_dyn(P, K.dyn, S, i, ring_slot, row);
+    } else if (P.n_dyn > 0) {
+        ring_store(P, S, i, ring_slot, dyn_rp, e.pos_idx);
+    }
     acc.sum_rew = dadd(acc.sum_rew, rew);
     if (done || trunc) {                                                     // :269-271 calculate_metrics
         acc.episodes += 1;
@@ -197,9 +210,10 @@ __device__ __forceinline__ StepThreadOut step_env(const GteParams& P, const GteD
         acc.sum_pr = dadd(acc.sum_pr, dsub(ddiv(val, P.v0), 1.0));           // :282
         acc.sum_mr = dadd(acc.sum_mr, dsub(ddiv(p1, __ldg(price + e.ep_start)), 1.0));   // :281
         if (autoreset) {
-            reset_env(P, D, S, i, tick, ring_slot, e);                       // in-place auto-reset
+            reset_env<GEN>(P, D, S, i, tick, ring_slot, e, K.dyn);           // in-place auto-reset
             idx = e.ep_start;
             dyn_pos = dyn_rp = (float)pos_tab[e.pos_idx];                // first row: (position, position) :191-192
+            dyn_pr = dyn_rew = dyn_prog = 0.0f;
             if (P.n_datasets > 1) S.dataset_idx[i] = e.ds;
         }
     }
@@ -208,10 +222,12 @@ __device__ __forceinline__ StepThreadOut step_env(const GteParams& P, const GteD
     StepThreadOut r;
     r.idx = idx; r.ep_start = e.ep_start; r.ds = e.ds;
     r.dyn_pos = dyn_pos; r.dyn_rp = dyn_rp;
+    r.dyn_pr = dyn_pr; r.dyn_rew = dyn_rew; r.dyn_prog = dyn_prog;
     return r;
 }
 
 // load + transition of env i in one go (fused step+gather kernel)
+template <bool GEN = false>
 __device__ __forceinline__ StepThreadOut step_env_now(const GteParams& P, const GteData& D, const GteState& S,
                                                       const void* __restrict__ actions, const StepConsts& K,
                                                       const GteStepOut& O, uint64_t tick, int ring_slot, int autoreset,
@@ -219,7 +235,7 @@ __device__ __forceinline__ StepThreadOut step_env_now(const GteParams& P, const 
     const EnvIn in = load_env(P, D, S, actions, K, i);
     double p0, p1;
     load_prices(P, D, in, p0, p1);
-    return step_env(P, D, S, K, O, tick, ring_slot, autoreset, i, in, p0, p1, acc, pos_tab);
+    return step_env<true, GEN>(P, D, S, K, O, tick, ring_slot, autoreset, i, in, p0, p1, acc, pos_tab);
 }
 
 // The one-row observations (windows=None, environments.py:156-157) of the 32 consecutive envs of a warp; every lane of
@@ -230,6 +246,12 @@ __device__ __forceinline__ StepThreadOut step_env_now(const GteParams& P, const 
 //                      fetching (row, dataset, dynamic features) of the owning env by shuffle -> full 128-byte stores.
 //                      For MAPPED HOST memory, where every partial-sector store is its own PCIe transaction
 //                      (4096 envs: 60 us -> 27 us per host step).
+// GEN: dynamic columns in P.dyn_kinds order (general catalogue), else the default pair.
+__device__ __forceinline__ float dyn_value(const StepThreadOut& r, uint32_t kind) {
+    return kind == GTE_DYN_POSITION ? r.dyn_pos : kind == GTE_DYN_REAL_POSITION ? r.dyn_rp
+         : kind == GTE_DYN_PORTFOLIO_RETURN ? r.dyn_pr : kind == GTE_DYN_REWARD ? r.dyn_rew : r.dyn_prog;
+}
+template <bool GEN = false>
 __device__ __forceinline__ void write_obs_rows(const GteParams& P, const GteData& D, float* __restrict__ obs_rows, int64_t i,
                                                bool valid, const StepThreadOut& r, bool coalesced) {
     const int F = P.n_static + P.n_dyn;
@@ -238,7 +260,11 @@ __device__ __forceinline__ void write_obs_rows(const GteParams& P, const GteData
             const float* __restrict__ f = D.features + ((int64_t)r.ds * P.t_stride + r.idx) * P.n_static;
             float* __restrict__ o = obs_rows + i * F;
             for (int c = 0; c < P.n_static; ++c) o[c] = __ldg(f + c);
-            if (P.n_dyn > 0) { o[P.n_static] = r.dyn_pos; o[P.n_static + 1] = r.dyn_rp; }
+            if (GEN) {
+                for (int j = 0; j < P.n_dyn; ++j) o[P.n_static + j] = dyn_value(r, ((uint32_t)P.dyn_kinds >> (4 * j)) & 15u);
+            } else if (P.n_dyn > 0) {
+                o[P.n_static] = r.dyn_pos; o[P.n_static + 1] = r.dyn_rp;
+            }
         }
         return;
     }
@@ -250,8 +276,18 @@ __device__ __forceinline__ void write_obs_rows(const GteParams& P, const GteData
         const int idx = __shfl_sync(FULL, r.idx, e), ds = __shfl_sync(FULL, r.ds, e);
         const float dp = __shfl_sync(FULL, r.dyn_pos, e), dr = __shfl_sync(FULL, r.dyn_rp, e);
         const bool ok = __shfl_sync(FULL, (int)valid, e) != 0;
-        if (ok) o[j] = c < P.n_static ? __ldg(D.features + ((int64_t)ds * P.t_stride + idx) * P.n_static + c)
-                                      : (c == P.n_static ? dp : dr);
+        if (GEN) {
+            StepThreadOut q;
+            q.dyn_pos = dp; q.dyn_rp = dr;
+            q.dyn_pr = __shfl_sync(FULL, r.dyn_pr, e);
+            q.dyn_rew = __shfl_sync(FULL, r.dyn_rew, e);
+            q.dyn_prog = __shfl_sync(FULL, r.dyn_prog, e);
+            if (ok) o[j] = c < P.n_static ? __ldg(D.features + ((int64_t)ds * P.t_stride + idx) * P.n_static + c)
+                                          : dyn_value(q, ((uint32_t)P.dyn_kinds >> (4 * (c - P.n_static))) & 15u);
+        } else {
+            if (ok) o[j] = c < P.n_static ? __ldg(D.features + ((int64_t)ds * P.t_stride + idx) * P.n_static + c)
+                                          : (c == P.n_static ? dp : dr);
+        }
     }
 }
 

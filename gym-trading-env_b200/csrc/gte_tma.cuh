@@ -15,6 +15,7 @@ struct ObsShape {
     uint32_t magicF;             // ceil(2^32 / F)
     int row_bytes, win_bytes, n_vec;
     int w_mask;                  // W-1 when W is a power of two, else -1
+    DynLayout dyn;               // dynamic-column descriptor: which ring block each dynamic column reads
 };
 
 static inline ObsShape make_shape(const GteParams& P) {
@@ -28,6 +29,7 @@ static inline ObsShape make_shape(const GteParams& P) {
     s.win_bytes = s.W * s.row_bytes;
     s.n_vec = s.win_bytes / 16;
     s.w_mask = (s.W & (s.W - 1)) == 0 ? s.W - 1 : -1;
+    s.dyn = dyn_layout(P);
     return s;
 }
 

@@ -22,6 +22,8 @@ import numpy as np
 import torch
 
 from . import _cabi
+from .dynamic_features import (DeviceFeature, episode_progress_feature, parse_dynamic_features,  # noqa: F401
+                               portfolio_return_feature, reward_feature)
 from .data import SeriesArrays, build_window_tables, frame_to_arrays, load_frame, reconcile_series
 
 
@@ -293,9 +295,11 @@ class TradingVectorEnv(_VectorEnvBase):
     are widened by the step kernel's own load — lossless, 8x fewer host-to-device bytes than gymnasium's int64.
 
     ``reward_function`` must be :func:`basic_reward_function` or a :class:`DeviceReward` from the fused
-    catalogue (log / simple return with scale and clip), and ``dynamic_feature_functions`` the two
-    defaults or ``[]``: arbitrary Python callbacks over a History cannot run inside the kernel and
-    there is deliberately no CPU fallback (NotImplementedError).
+    catalogue (log / simple return with scale and clip), and ``dynamic_feature_functions`` a list of up to five
+    :class:`DeviceFeature` columns, each kind at most once, in any order (``position``, ``real_position`` — also
+    spelled :func:`dynamic_feature_last_position_taken` / :func:`dynamic_feature_real_position` —
+    ``portfolio_return``, ``reward``, ``episode_progress``; see ``dynamic_features.py``): arbitrary Python callbacks
+    over a History cannot run inside the kernel and there is deliberately no CPU fallback (NotImplementedError).
 
     Returned tensors are persistent buffers overwritten by the next call: copy what you keep.
     """
@@ -342,13 +346,7 @@ class TradingVectorEnv(_VectorEnvBase):
                 "callbacks over a History cannot run inside the CUDA step kernel and there is no CPU fallback")
         self.reward_function = reward_function
         dyn = list(dynamic_feature_functions)
-        if len(dyn) == 0:
-            self._n_dyn = 0
-        elif [_fn_name(f) for f in dyn] == ["dynamic_feature_last_position_taken", "dynamic_feature_real_position"]:
-            self._n_dyn = 2
-        else:
-            raise NotImplementedError(
-                "dynamic_feature_functions must be the two defaults (environments.py:20-24, :82) or []")
+        self._n_dyn, self._dyn_kinds = parse_dynamic_features(dyn, max_episode_duration)
         self.dynamic_feature_functions = dyn
         if not (1 <= len(self.positions) <= _cabi.GTE_MAX_POSITIONS):
             raise ValueError(f"between 1 and {_cabi.GTE_MAX_POSITIONS} positions are supported")
@@ -490,9 +488,11 @@ class TradingVectorEnv(_VectorEnvBase):
         self._pos_idx, self._step, self._ep_start, self._dataset_idx = i32(N), i32(N), i32(N), i32(N)
         self._plan_cursor, self._ds_episodes = i32(N), i32(N)
         self._ds_used = torch.zeros(N, dtype=torch.int64, device=dev)
-        # dynamic-feature ring: one GTE_RING_TILE_BYTES(W) block per tile of 32 envs, slots indexed by the
+        # dynamic-feature ring: one GTE_RING_TILE_BYTES_DYN block per tile of 32 envs, slots indexed by the
         # device-resident iteration clock (layout: include/gte_b200.h)
-        self._dyn_ring = torch.zeros((N + 31) // 32, W * 160, dtype=torch.uint8, device=dev)
+        # (unused without dynamic columns: then sized as for the default pair, the shape state_dict() has always had)
+        tile = _cabi.ring_tile_bytes(W, self._n_dyn or 2, self._dyn_kinds)
+        self._dyn_ring = torch.zeros((N + 31) // 32, tile, dtype=torch.uint8, device=dev)
         self._ring_clock = torch.zeros(1, dtype=torch.int64, device=dev)
         self._error_flag = i32(1)
         self._tick_dev = torch.zeros(1, dtype=torch.int64, device=dev)
@@ -532,7 +532,7 @@ class TradingVectorEnv(_VectorEnvBase):
         p = _cabi.GteParams()
         p.n_envs, p.n_positions = self.num_envs, len(self.positions)
         p.windows = 0 if self.windows is None else int(self.windows)
-        p.n_static, p.n_dyn = self._n_static, self._n_dyn
+        p.n_static, p.n_dyn, p.dyn_kinds = self._n_static, self._n_dyn, self._dyn_kinds
         p.max_episode_duration = -1 if self.max_episode_duration == "max" else int(self.max_episode_duration)
         p.n_datasets = self._n_ds
         p.initial_position_idx = -1 if self.initial_position == "random" else self.positions.index(self.initial_position)

@@ -41,6 +41,14 @@ extern "C" {
 #define GTE_RING_BYTES(N, W) ((((int64_t)(N) + 31) / 32) * GTE_RING_TILE_BYTES(W))
 #define GTE_RING_RP_OFFSET(s, e) ((s) * 128 + (((((e) >> 2) ^ ((s) & 7))) << 4) + (((e) & 3) << 2))
 #define GTE_RING_POS_OFFSET(W, s, e) ((W) * 128 + (s) * 32 + (e))
+/* The same layout for any dynamic-feature catalogue (GteParams.dyn_kinds): n_f32 blocks of W rows x 32 f32 values, one
+ * per f32 kind, then n_pos (0 or 1) blocks of W rows x 32 u8 position indices.  With n_f32 = n_pos = 1 these are byte
+ * for byte GTE_RING_TILE_BYTES / GTE_RING_RP_OFFSET / GTE_RING_POS_OFFSET. */
+#define GTE_MAX_DYN 5
+#define GTE_RING_TILE_BYTES_DYN(W, n_f32, n_pos) ((W) * (128 * (n_f32) + 32 * (n_pos)))
+#define GTE_RING_BYTES_DYN(N, W, n_f32, n_pos) ((((int64_t)(N) + 31) / 32) * GTE_RING_TILE_BYTES_DYN(W, n_f32, n_pos))
+#define GTE_RING_F32_OFFSET(W, k, s, e) ((k) * (W) * 128 + GTE_RING_RP_OFFSET(s, e))
+#define GTE_RING_POS_OFFSET_DYN(W, n_f32, s, e) ((n_f32) * (W) * 128 + (s) * 32 + (e))
 #define GTE_STEP_THREADS 256       /* envs per tile of the step kernel */
 #define GTE_MAX_PARTIAL_ROWS 4096  /* rows of GteStepOut.metric_partials (one per CTA; every grid is capped at this) */
 /* Result block of gte_step_host — everything a host policy needs back from one iteration, in ONE piece of memory
@@ -89,6 +97,17 @@ enum GteRewardKind {
     GTE_REWARD_SIMPLE_RETURN = 1   /* f = (v_t - v_{t-1}) / v_{t-1}                                         */
 };
 
+/* Dynamic-feature kinds (GteParams.dyn_kinds): the device catalogue standing in for the reference's
+ * `dynamic_feature_functions` (environments.py:43-48, :153-154).  Each column is the fp64 value cast to float32;
+ * in an episode's first row (the reset row, :191-192) position and real_position read the position, the others 0. */
+enum GteDynKind {
+    GTE_DYN_POSITION = 1,          /* history["position", -1]            (:20-21; u8 position index in the ring) */
+    GTE_DYN_REAL_POSITION = 2,     /* history["real_position", -1]       (:23-24)                                */
+    GTE_DYN_PORTFOLIO_RETURN = 3,  /* history["portfolio_valuation", -1] / history["portfolio_valuation", 0] - 1 */
+    GTE_DYN_REWARD = 4,            /* history["reward", -1]: the step's reward (0 when terminated)               */
+    GTE_DYN_EPISODE_PROGRESS = 5   /* history["step", -1] / max_episode_duration                                 */
+};
+
 enum GteErrorBit {
     GTE_E_ACTION_RANGE = 1, GTE_E_PAST_END = 2, GTE_E_PLAN_RANGE = 4, GTE_E_PLAN_EXHAUSTED = 8, GTE_E_NEGATIVE_ACTION = 16
 };
@@ -108,7 +127,7 @@ typedef struct GteParams {
     int32_t n_positions;             /* len(positions)  (:98, action space Discrete(P) :112)           */
     int32_t windows;                 /* `windows` (:101); 0 = None                                     */
     int32_t n_static;                /* static "feature*" columns (:130)                               */
-    int32_t n_dyn;                   /* 0 or 2: the default dynamic features (:20-24, :82)             */
+    int32_t n_dyn;                   /* dynamic feature columns, 0..GTE_MAX_DYN (see dyn_kinds)          */
     int32_t max_episode_duration;    /* (:94) -1 = 'max'                                               */
     int32_t n_datasets;              /* 1 for TradingEnv                                               */
     int32_t initial_position_idx;    /* index into positions, -1 = 'random' (:105, :167)               */
@@ -122,7 +141,10 @@ typedef struct GteParams {
                                         host->device bytes of a host policy 8x and are widened in the step kernel's load */
     int32_t strict_actions;          /* 1: any negative action other than -1 sets error bit 4 (still treated as hold).
                                         The reference's positions[-k] would index from the END of the list (:234)        */
-    int32_t reserved0;
+    int32_t dyn_kinds;               /* enum GteDynKind of dynamic column j in bits 4j..4j+3, each kind at most once.
+                                        0 = the defaults: n_dyn == 0 none, n_dyn == 2 (position, real_position)
+                                        (:20-24, :82), the same descriptor as the explicit 0x21.  episode_progress
+                                        needs max_episode_duration > 0                                           */
     int64_t t_stride;                /* rows allocated per dataset in `price` / `features`             */
     int64_t env_id_offset;           /* global index of env 0 (multi-GPU sharding; keys the RNG)       */
     uint64_t seed;                   /* Philox key                                                     */
@@ -164,13 +186,15 @@ typedef struct GteState {
     /* Dynamic-feature ring, indexed by TIME: the row an env observed at lockstep iteration c (c = *ring_clock,
      * advanced by every gte_step / gte_step_obs call) lives in slot c % W, W = max(windows,1); a window reads slots
      * c-W+1 .. c, and its rows before ep_start read as zero (the env was reset less than W iterations ago).
-     * Memory: one contiguous block of GTE_RING_TILE_BYTES(W) per tile of 32 consecutive envs, so that the gather
-     * fetches a tile's whole ring with one bulk copy while one iteration's stores are a full 128-byte line + a
-     * full 32-byte sector per warp.  Inside a block: W rows of 32 f32 real_position values (:24) — env lane e of
-     * slot s at GTE_RING_RP_OFFSET(s, e), 16-byte chunks XOR-swizzled by the slot so that column reads from
-     * shared memory spread over the banks — then W rows of 32 u8 position INDICES at GTE_RING_POS_OFFSET(W, s, e)
-     * (the dynamic feature "position" is float32(positions[index]), :20-21). */
-    uint8_t* dyn_ring;               /* u8 [GTE_RING_BYTES(N, W)], 16-byte aligned                               */
+     * Memory: one contiguous block per tile of 32 consecutive envs, so that the gather fetches a tile's whole ring
+     * with one bulk copy while one iteration's stores are a full 128-byte line (+ a full 32-byte sector) per warp
+     * and column.  Inside a block: for each configured f32 kind, in kind-code order (real_position, portfolio_return,
+     * reward, episode_progress), W rows of 32 f32 values — f32 block k, env lane e of slot s at
+     * GTE_RING_F32_OFFSET(W, k, s, e), 16-byte chunks XOR-swizzled by the slot so that column reads from shared memory
+     * spread over the banks — then, when "position" is configured, W rows of 32 u8 position INDICES at
+     * GTE_RING_POS_OFFSET_DYN(W, n_f32, s, e) (the feature is float32(positions[index]), :20-21).  The default pair is
+     * GTE_RING_TILE_BYTES(W) per tile with real_position at GTE_RING_RP_OFFSET and the indices at GTE_RING_POS_OFFSET. */
+    uint8_t* dyn_ring;               /* u8 [GTE_RING_BYTES_DYN(N, W, n_f32, n_pos)], 16-byte aligned; unused when n_dyn == 0 */
     uint64_t* ring_clock;            /* u64 [1]  lockstep iterations so far, advanced ON THE DEVICE              */
     int32_t* plan_cursor;            /* i32 [N]  next episode slot of reset_plan                       */
     uint64_t* ds_used;               /* u64 [N]  datasets used in the current rotation round (:383)    */
@@ -306,7 +330,7 @@ int gte_step(const GteParams* params, const GteData* data, const GteState* state
 
 /* Replaces TradingEnv._get_obs (environments.py:152-160): obs f32 [N, F] (windows=None) or
  * [N, W, F], F = n_static + n_dyn; static columns gathered from the device-resident tables,
- * dynamic columns from the dynamic-feature ring. */
+ * dynamic columns (in dyn_kinds order) from the dynamic-feature ring; window rows before the episode start are 0. */
 int gte_gather_obs(const GteParams* params, const GteData* data, const GteState* state,
                    float* obs, int variant, void* stream);
 
