@@ -144,25 +144,16 @@ __device__ __forceinline__ int next_dataset(const GteParams& P, const GteState& 
 
 // Dynamic-feature ring (time-indexed, one block per 32-env tile: include/gte_b200.h): the row env i observes at
 // lockstep iteration c lives in slot c % W.  All envs write the same slot in one iteration: a warp stores one
-// full 128-byte line of real_position values and one full 32-byte sector of position indices.
+// full 128-byte line per f32 column and one full 32-byte sector of position indices.
 __device__ __forceinline__ int ring_slot_of(const GteParams& P, uint64_t clock) {
     const int W = P.windows > 0 ? P.windows : 1;
     return (int)(clock % (uint64_t)W);
 }
-__device__ __forceinline__ const uint8_t* ring_tile(const GteState& S, int W, int64_t env) {
-    return S.dyn_ring + (env >> 5) * (int64_t)GTE_RING_TILE_BYTES(W);
-}
-__device__ __forceinline__ void ring_store(const GteParams& P, const GteState& S, int i, int slot, float rp, int pos_idx) {
-    const int W = P.windows > 0 ? P.windows : 1;
-    const int e = i & 31;
-    uint8_t* tile = S.dyn_ring + (int64_t)(i >> 5) * GTE_RING_TILE_BYTES(W);
-    *reinterpret_cast<float*>(tile + GTE_RING_RP_OFFSET(slot, e)) = rp;
-    tile[GTE_RING_POS_OFFSET(W, slot, e)] = (uint8_t)pos_idx;
-}
 
 // Dynamic-column descriptor, derived once on the host from (n_dyn, dyn_kinds) by dyn_layout(): drives the ring layout
 // (include/gte_b200.h, GteState.dyn_ring) on both the step and the gather side.  `general` is false for no dynamic
-// columns and for the default pair (position, real_position): those run the kernels' original instantiations.
+// columns and for the default pair (position, real_position): those run the GEN = false instantiations, whose layout
+// is known at compile time (RingLayout).
 constexpr uint32_t kDynPosBlock = 0xF, kDynNone = 0xE;
 struct DynLayout {
     uint32_t col_src;     // nibble j: the ring block column j reads: f32 block 0..3, or kDynPosBlock (u8 position indices)
@@ -170,6 +161,31 @@ struct DynLayout {
     int n_f32, n_pos;     // f32 blocks, position-index blocks (0 or 1)
     int tile_bytes;       // GTE_RING_TILE_BYTES_DYN(W, n_f32, n_pos)
     bool general;
+};
+
+// The ring layout as the kernels see it, and the only code that branches on GEN to describe it.  GEN = false: the
+// default pair, every answer a compile-time constant (column 0 reads the position-index block, column 1 f32 block 0;
+// per-column answers fold by column index, which keeps the pair's registers where a decoded constant descriptor would
+// not).  GEN = true: the general catalogue, answers read from L.  Kernels that may run without dynamic columns check
+// n_dyn > 0 before they touch the ring.
+template <bool GEN>
+struct RingLayout {
+    const DynLayout& L;
+    __device__ __forceinline__ int n_cols() const { return GEN ? L.n_f32 + L.n_pos : 2; }
+    __device__ __forceinline__ bool is_pos(int j) const { return GEN ? ((L.col_src >> (4 * j)) & 15u) == kDynPosBlock : j == 0; }
+    __device__ __forceinline__ int f32_block(int j) const { return GEN ? (int)((L.col_src >> (4 * j)) & 15u) : 0; }
+    // f32 block of kind k, kDynPosBlock for position, or kDynNone when the kind is not configured
+    __device__ __forceinline__ uint32_t kind_block(int k) const {
+        return GEN ? (L.kind_blk >> (4 * k)) & 15u
+                   : (k == GTE_DYN_POSITION ? kDynPosBlock : k == GTE_DYN_REAL_POSITION ? 0u : kDynNone);
+    }
+    __device__ __forceinline__ int n_f32() const { return GEN ? L.n_f32 : 1; }
+    __device__ __forceinline__ int n_pos() const { return GEN ? L.n_pos : 1; }
+    __device__ __forceinline__ int tile_bytes(int W) const { return GEN ? L.tile_bytes : GTE_RING_TILE_BYTES_DYN(W, 1, 1); }
+    // the ring block of the 32-env tile that holds env
+    __device__ __forceinline__ const uint8_t* tile_of(const uint8_t* ring, int W, int64_t env) const {
+        return ring + (env >> 5) * (int64_t)tile_bytes(W);
+    }
 };
 
 // dyn_kinds with the legacy 0 spelled out (n_dyn == 2: the default pair, 0x21)
@@ -198,25 +214,40 @@ static inline DynLayout dyn_layout(const GteParams& P) {
     return L;
 }
 
-__device__ __forceinline__ uint32_t dyn_block_of(const DynLayout& L, int kind) { return (L.kind_blk >> (4 * kind)) & 15u; }
-
-// One row of every configured dynamic column (general catalogue), fp64 values already cast to f32 as numpy casts (:154).
+// One row of every dynamic column, fp64 values already cast to f32 as numpy casts (:154); the kinds that are not
+// configured are ignored.
 struct DynRow {
     float rp, pr, rew, prog;      // real_position, portfolio_return, reward, episode_progress
     int pos_idx;                  // position: index into positions
 };
-__device__ __forceinline__ void ring_store_dyn(const GteParams& P, const DynLayout& L, const GteState& S, int i, int slot,
-                                               const DynRow& r) {
+// Writes row r of env i into ring slot `slot` (step and reset side); needs n_dyn > 0.
+template <bool GEN>
+__device__ __forceinline__ void ring_store(const GteParams& P, const DynLayout& L, const GteState& S, int i, int slot,
+                                           const DynRow& r) {
+    const RingLayout<GEN> R{L};
     const int W = P.windows > 0 ? P.windows : 1;
     const int e = i & 31;
-    uint8_t* tile = S.dyn_ring + (int64_t)(i >> 5) * L.tile_bytes;
+    uint8_t* tile = S.dyn_ring + (int64_t)(i >> 5) * R.tile_bytes(W);
     const float v[4] = {r.rp, r.pr, r.rew, r.prog};
 #pragma unroll
     for (int k = GTE_DYN_REAL_POSITION; k <= GTE_DYN_EPISODE_PROGRESS; ++k) {
-        const uint32_t b = dyn_block_of(L, k);
+        const uint32_t b = R.kind_block(k);
         if (b < kDynNone) *reinterpret_cast<float*>(tile + GTE_RING_F32_OFFSET(W, (int)b, slot, e)) = v[k - GTE_DYN_REAL_POSITION];
     }
-    if (L.n_pos) tile[GTE_RING_POS_OFFSET_DYN(W, L.n_f32, slot, e)] = (uint8_t)r.pos_idx;
+    if (R.n_pos()) tile[GTE_RING_POS_OFFSET_DYN(W, R.n_f32(), slot, e)] = (uint8_t)r.pos_idx;
+}
+
+// Dynamic column j of env lane e in ring slot s of a ring tile (the gathers' read).  CG: a global-memory tile read
+// through L2 only, as the vec gather reads the ring.
+template <bool GEN, bool CG = false>
+__device__ __forceinline__ float ring_value(const GteParams& P, const RingLayout<GEN>& R, int W, const uint8_t* tile,
+                                            int j, int s, int e) {
+    if (R.is_pos(j)) {
+        const uint8_t* p = tile + GTE_RING_POS_OFFSET_DYN(W, R.n_f32(), s, e);
+        return (float)P.positions[CG ? __ldcg(p) : *p];           // fp64 -> fp32 as numpy casts (:154)
+    }
+    const float* p = reinterpret_cast<const float*>(tile + GTE_RING_F32_OFFSET(W, R.f32_block(j), s, e));
+    return CG ? __ldcg(p) : *p;
 }
 
 struct EnvRegs {          // the per-env state a step keeps in registers
@@ -226,7 +257,7 @@ struct EnvRegs {          // the per-env state a step keeps in registers
 
 // TradingEnv.reset (environments.py:163-199) preceded by MultiDatasetTradingEnv.reset (:393-400).
 // Rare path (once per episode): plan/rotation bookkeeping goes straight to global memory.
-// GEN: the general dynamic-feature catalogue (L.general), else no dynamic columns or the default pair.
+// GEN: the general dynamic-feature catalogue (L.general), else no dynamic columns or the default pair (RingLayout).
 template <bool GEN = false>
 __device__ __forceinline__ void reset_env(const GteParams& P, const GteData& D, const GteState& S,
                                        int i, uint64_t tick, int ring_slot, EnvRegs& e, const DynLayout& L) {
@@ -278,11 +309,9 @@ __device__ __forceinline__ void reset_env(const GteParams& P, const GteData& D, 
     e.pf = target_portfolio(position, P.v0, price);                          // :179-183
     for (int k = 0; k < P.n_limit_positions; ++k)                            // self._limit_orders = {} (:168)
         S.limit_price[(int64_t)i * P.n_positions + S.limit_seq[k]] = __longlong_as_double(0x7ff8000000000000ll);
-    if (GEN) {                                // first obs row (:191-192): position, real_position = position, else 0
+    if (P.n_dyn > 0) {                        // first obs row (:191-192): position, real_position = position, else 0
         const DynRow r = {(float)position, 0.0f, 0.0f, 0.0f, e.pos_idx};
-        ring_store_dyn(P, L, S, i, ring_slot, r);
-    } else if (P.n_dyn > 0) {                                                // first obs row: (position, position) :191-192
-        ring_store(P, S, i, ring_slot, (float)position, e.pos_idx);
+        ring_store<GEN>(P, L, S, i, ring_slot, r);
     }
 }
 

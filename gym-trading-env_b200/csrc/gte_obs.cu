@@ -18,24 +18,9 @@
 
 namespace gte {
 
-// One dynamic column of the general catalogue (GEN instantiations): column j of env lane e in ring slot s of a tile
-// (CG: a global-memory tile read through L2 only, as the vec gather reads the ring).
-template <bool CG = false>
-__device__ __forceinline__ float dyn_ring_value(const GteParams& P, const ObsShape& sh, const uint8_t* tile, int j, int s, int e) {
-    const uint32_t src = (sh.dyn.col_src >> (4 * j)) & 15u;
-    if (src == kDynPosBlock) {
-        const uint8_t* p = tile + GTE_RING_POS_OFFSET_DYN(sh.W, sh.dyn.n_f32, s, e);
-        return (float)P.positions[CG ? __ldcg(p) : *p];
-    }
-    const float* p = reinterpret_cast<const float*>(tile + GTE_RING_F32_OFFSET(sh.W, (int)src, s, e));
-    return CG ? __ldcg(p) : *p;
-}
-__device__ __forceinline__ const uint8_t* ring_tile_dyn(const GteState& S, const ObsShape& sh, int64_t env) {
-    return S.dyn_ring + (env >> 5) * (int64_t)sh.dyn.tile_bytes;
-}
-
 // ------------------------------------------------------------------------------------------ generic
-// GEN (every kernel below): dynamic columns of the general catalogue (sh.dyn), else none or the default pair.
+// GEN (every kernel below): dynamic columns of the general catalogue (sh.dyn), else none or the default pair, whose ring
+// layout is known at compile time (RingLayout).
 template <int G, bool GEN = false>
 __global__ void __launch_bounds__(256)
 obs_generic_kernel(const GteParams P, const GteData D, const GteState S, float* __restrict__ obs,
@@ -44,6 +29,7 @@ obs_generic_kernel(const GteParams P, const GteData D, const GteState S, float* 
     const int lane = threadIdx.x % G;
     const int64_t n_groups = (int64_t)gridDim.x * groups_per_block;
     const int per_env = sh.W * sh.F;
+    const RingLayout<GEN> R{sh.dyn};
     const int s0 = sh.nd > 0 ? (int)((*S.ring_clock + 1ull) % (uint64_t)sh.W) : 0;    // ring slot of window row 0
     for (int64_t env = env_begin + (int64_t)blockIdx.x * groups_per_block + threadIdx.x / G; env < env_end;
          env += n_groups) {
@@ -63,14 +49,8 @@ obs_generic_kernel(const GteParams P, const GteData D, const GteState S, float* 
                 int slot = s0 + w;
                 if (slot >= sh.W) slot -= sh.W;
                 const int e32 = (int)(env & 31);
-                if (GEN) {
-                    v = (r < ep_start) ? 0.0f : dyn_ring_value(P, sh, ring_tile_dyn(S, sh, env), c - sh.ns, slot, e32);
-                } else {
-                    const uint8_t* __restrict__ ring = ring_tile(S, sh.W, env);
-                    v = (r < ep_start) ? 0.0f
-                      : (c == sh.ns ? (float)P.positions[ring[GTE_RING_POS_OFFSET(sh.W, slot, e32)]]
-                                    : *reinterpret_cast<const float*>(ring + GTE_RING_RP_OFFSET(slot, e32)));
-                }
+                const uint8_t* __restrict__ ring = R.tile_of(S.dyn_ring, sh.W, env);
+                v = (r < ep_start) ? 0.0f : ring_value(P, R, sh.W, ring, c - sh.ns, slot, e32);
             }
             out[e] = v;
         }
@@ -96,6 +76,7 @@ obs_vec_kernel(const GteParams P, const GteData D, const GteState S, float* __re
                const ObsShape sh, const int env_begin, const int env_end) {
     const int lane = threadIdx.x & 31;
     const int64_t n_warps = (int64_t)gridDim.x * (blockDim.x >> 5);
+    const RingLayout<GEN> R{sh.dyn};
     const int s0 = sh.nd > 0 ? (int)((*S.ring_clock + 1ull) % (uint64_t)sh.W) : 0;    // ring slot of window row 0
     for (int64_t env = env_begin + (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); env < env_end;
          env += n_warps) {
@@ -104,7 +85,7 @@ obs_vec_kernel(const GteParams P, const GteData D, const GteState S, float* __re
         const int ds = S.dataset_idx[env];
         const int r0 = idx + 1 - sh.W;
         const char* __restrict__ src = window_src(D, sh, ds, r0);
-        const uint8_t* __restrict__ ring = GEN ? ring_tile_dyn(S, sh, env) : ring_tile(S, sh.W, env);
+        const uint8_t* __restrict__ ring = R.tile_of(S.dyn_ring, sh.W, env);
         const int e32 = (int)(env & 31);
         char* __restrict__ dst = reinterpret_cast<char*>(obs) + env * (int64_t)sh.win_bytes;
         for (int j = lane; j < sh.n_vec; j += 32) {
@@ -120,19 +101,12 @@ obs_vec_kernel(const GteParams P, const GteData D, const GteState S, float* __re
                         const int r = r0 + w;
                         int slot = s0 + w;
                         if (slot >= sh.W) slot -= sh.W;
-                        if (GEN) {
-                            pv[k] = (r < ep_start) ? 0.0f : dyn_ring_value<true>(P, sh, ring, c - sh.ns, slot, e32);
-                            continue;
-                        }
-                        const uint8_t* rpos = ring + GTE_RING_POS_OFFSET(sh.W, slot, e32);
-                        const float* rrp = reinterpret_cast<const float*>(ring + GTE_RING_RP_OFFSET(slot, e32));
-                        if (PAIR) {
+                        if (PAIR) {                      // c == sh.ns: columns 0 and 1 at once
                             const bool live = r >= ep_start;
-                            pv[k] = live ? (float)P.positions[__ldcg(rpos)] : 0.0f;
-                            pv[k + 1] = live ? __ldcg(rrp) : 0.0f;
+                            pv[k] = live ? ring_value<GEN, true>(P, R, sh.W, ring, 0, slot, e32) : 0.0f;
+                            pv[k + 1] = live ? ring_value<GEN, true>(P, R, sh.W, ring, 1, slot, e32) : 0.0f;
                         } else {
-                            pv[k] = (r < ep_start) ? 0.0f
-                                  : (c == sh.ns ? (float)P.positions[__ldcg(rpos)] : __ldcg(rrp));
+                            pv[k] = (r < ep_start) ? 0.0f : ring_value<GEN, true>(P, R, sh.W, ring, c - sh.ns, slot, e32);
                         }
                     }
                 }
@@ -222,8 +196,9 @@ obs_tma_coop_kernel(const GteParams P, const GteData D, const GteState S, float*
     const bool ring = sh.nd > 0;
     const uint32_t win_bytes = (uint32_t)sh.win_bytes;
     const uint32_t wstage_bytes = win_bytes * G;
-    const uint32_t rstride = GEN ? (uint32_t)sh.dyn.tile_bytes : (uint32_t)GTE_RING_TILE_BYTES(sh.W);
-    auto ring_src = [&](int64_t env) -> const uint8_t* { return GEN ? ring_tile_dyn(S, sh, env) : ring_tile(S, sh.W, env); };
+    const RingLayout<GEN> R{sh.dyn};
+    const uint32_t rstride = (uint32_t)R.tile_bytes(sh.W);
+    auto ring_src = [&](int64_t env) -> const uint8_t* { return R.tile_of(S.dyn_ring, sh.W, env); };
     unsigned char* rbase = smem_raw;
     unsigned char* wbase = rbase + (ring ? (size_t)RT * rstride : 0);
 
@@ -472,12 +447,7 @@ obs_tma_coop_kernel(const GteParams P, const GteData D, const GteState S, float*
                             if (w < 0) w += sh.W;
                             if (w >= live0) {                    // rows before the episode start stay zero
                                 float* qd = fbuf + w * sh.F + sh.ns;
-                                if (GEN) {
-                                    for (int j = 0; j < sh.nd; ++j) qd[j] = dyn_ring_value(P, sh, rtile, j, s, e);
-                                } else {
-                                    qd[0] = (float)P.positions[rtile[GTE_RING_POS_OFFSET(sh.W, s, e)]];   // fp64 -> fp32 as numpy casts (:154)
-                                    qd[1] = *reinterpret_cast<const float*>(rtile + GTE_RING_RP_OFFSET(s, e));
-                                }
+                                for (int j = 0; j < R.n_cols(); ++j) qd[j] = ring_value(P, R, sh.W, rtile, j, s, e);
                             }
                         }
                     }
@@ -515,101 +485,63 @@ static size_t tma_smem_bytes(const ObsShape& sh, const TmaConfig& c) {
     return (size_t)c.group * c.wstages * sh.win_bytes + ring;
 }
 
-// The general dynamic-feature catalogue: the default pipeline shape (3 window stages, 2 ring tiles, the group sizes
-// tma_config() may pick) in every form.
-static ObsKernelFn tma_kernel_gen(int key, int unit, bool fused, bool dyn) {
-    if (dyn) {
-        if (fused || unit != kTileEnvs) return nullptr;
+// (window stages, ring-tile stages, envs per group) combinations compiled in: the default pipeline shape (3 window
+// stages, 2 ring tiles, the groups tma_config() may pick) in every form — work units of 32, 16 and 8 envs, the fused
+// step+gather form, the claimed-tiles form (large batches) — and, for no columns / the default pair, a few more
+// shapes for tuning runs (GTE_TMA_STAGES / _RTILES / _GROUP).
+template <bool GEN>
+static ObsKernelFn tma_kernel_of(int key, int unit, bool fused, bool dyn) {
+    if (dyn && !fused && unit == kTileEnvs) {
         switch (key) {
-            case 30201: return obs_tma_coop_kernel<3, 2, 1, 32, false, true, true>;
-            case 30202: return obs_tma_coop_kernel<3, 2, 2, 32, false, true, true>;
-            case 30204: return obs_tma_coop_kernel<3, 2, 4, 32, false, true, true>;
-            default: return nullptr;
+            case 30201: return obs_tma_coop_kernel<3, 2, 1, 32, false, true, GEN>;
+            case 30202: return obs_tma_coop_kernel<3, 2, 2, 32, false, true, GEN>;
+            case 30204: return obs_tma_coop_kernel<3, 2, 4, 32, false, true, GEN>;
         }
     }
-    switch ((fused ? 1000000 : 0) + unit * 100000 + key) {
-        case 3230201: return obs_tma_coop_kernel<3, 2, 1, 32, false, false, true>;
-        case 3230202: return obs_tma_coop_kernel<3, 2, 2, 32, false, false, true>;
-        case 3230204: return obs_tma_coop_kernel<3, 2, 4, 32, false, false, true>;
-        case 1630201: return obs_tma_coop_kernel<3, 2, 1, 16, false, false, true>;
-        case 1630202: return obs_tma_coop_kernel<3, 2, 2, 16, false, false, true>;
-        case 1630204: return obs_tma_coop_kernel<3, 2, 4, 16, false, false, true>;
-        case 830201: return obs_tma_coop_kernel<3, 2, 1, 8, false, false, true>;
-        case 830202: return obs_tma_coop_kernel<3, 2, 2, 8, false, false, true>;
-        case 830204: return obs_tma_coop_kernel<3, 2, 4, 8, false, false, true>;
-        case 4230201: return obs_tma_coop_kernel<3, 2, 1, 32, true, false, true>;
-        case 4230202: return obs_tma_coop_kernel<3, 2, 2, 32, true, false, true>;
-        case 4230204: return obs_tma_coop_kernel<3, 2, 4, 32, true, false, true>;
-        case 2630201: return obs_tma_coop_kernel<3, 2, 1, 16, true, false, true>;
-        case 2630202: return obs_tma_coop_kernel<3, 2, 2, 16, true, false, true>;
-        case 2630204: return obs_tma_coop_kernel<3, 2, 4, 16, true, false, true>;
-        case 1830201: return obs_tma_coop_kernel<3, 2, 1, 8, true, false, true>;
-        case 1830202: return obs_tma_coop_kernel<3, 2, 2, 8, true, false, true>;
-        case 1830204: return obs_tma_coop_kernel<3, 2, 4, 8, true, false, true>;
-        default: return nullptr;
+    if (!dyn) {
+        switch ((fused ? 1000000 : 0) + unit * 100000 + key) {
+            case 3230201: return obs_tma_coop_kernel<3, 2, 1, 32, false, false, GEN>;
+            case 3230202: return obs_tma_coop_kernel<3, 2, 2, 32, false, false, GEN>;
+            case 3230204: return obs_tma_coop_kernel<3, 2, 4, 32, false, false, GEN>;
+            case 1630201: return obs_tma_coop_kernel<3, 2, 1, 16, false, false, GEN>;
+            case 1630202: return obs_tma_coop_kernel<3, 2, 2, 16, false, false, GEN>;
+            case 1630204: return obs_tma_coop_kernel<3, 2, 4, 16, false, false, GEN>;
+            case 830201: return obs_tma_coop_kernel<3, 2, 1, 8, false, false, GEN>;
+            case 830202: return obs_tma_coop_kernel<3, 2, 2, 8, false, false, GEN>;
+            case 830204: return obs_tma_coop_kernel<3, 2, 4, 8, false, false, GEN>;
+            case 4230201: return obs_tma_coop_kernel<3, 2, 1, 32, true, false, GEN>;
+            case 4230202: return obs_tma_coop_kernel<3, 2, 2, 32, true, false, GEN>;
+            case 4230204: return obs_tma_coop_kernel<3, 2, 4, 32, true, false, GEN>;
+            case 2630201: return obs_tma_coop_kernel<3, 2, 1, 16, true, false, GEN>;
+            case 2630202: return obs_tma_coop_kernel<3, 2, 2, 16, true, false, GEN>;
+            case 2630204: return obs_tma_coop_kernel<3, 2, 4, 16, true, false, GEN>;
+            case 1830201: return obs_tma_coop_kernel<3, 2, 1, 8, true, false, GEN>;
+            case 1830202: return obs_tma_coop_kernel<3, 2, 2, 8, true, false, GEN>;
+            case 1830204: return obs_tma_coop_kernel<3, 2, 4, 8, true, false, GEN>;
+        }
     }
+    if constexpr (!GEN) {
+        if (!fused && unit == kTileEnvs) {
+            switch ((dyn ? 1000000 : 0) + key) {
+                case 1030208: return obs_tma_coop_kernel<3, 2, 8, 32, false, true>;
+                case 30208: return obs_tma_coop_kernel<3, 2, 8>;
+                case 30304: return obs_tma_coop_kernel<3, 3, 4>;
+                case 40204: return obs_tma_coop_kernel<4, 2, 4>;
+                case 40304: return obs_tma_coop_kernel<4, 3, 4>;
+                case 20204: return obs_tma_coop_kernel<2, 2, 4>;
+                case 40202: return obs_tma_coop_kernel<4, 2, 2>;
+                case 60202: return obs_tma_coop_kernel<6, 2, 2>;
+                case 60302: return obs_tma_coop_kernel<6, 3, 2>;
+                case 20208: return obs_tma_coop_kernel<2, 2, 8>;
+            }
+        }
+    }
+    return nullptr;
 }
 
 static ObsKernelFn tma_kernel(const TmaConfig& c, int unit = kTileEnvs, bool fused = false, bool dyn = false, bool gen = false) {
-    // (window stages, ring-tile stages, envs per group) combinations compiled in; smaller work units, the fused
-    // step+gather form and the claimed-tiles form (large batches) for the default shapes
     const int key = c.wstages * 10000 + c.rtiles * 100 + c.group;
-    if (gen) return tma_kernel_gen(key, unit, fused, dyn);
-    if (dyn) {
-        if (fused || unit != kTileEnvs) return nullptr;
-        switch (key) {
-            case 30201: return obs_tma_coop_kernel<3, 2, 1, 32, false, true>;
-            case 30202: return obs_tma_coop_kernel<3, 2, 2, 32, false, true>;
-            case 30204: return obs_tma_coop_kernel<3, 2, 4, 32, false, true>;
-            case 30208: return obs_tma_coop_kernel<3, 2, 8, 32, false, true>;
-            default: return nullptr;
-        }
-    }
-    if (fused) {
-        switch (unit * 100000 + key) {
-            case 3230201: return obs_tma_coop_kernel<3, 2, 1, 32, true>;
-            case 3230202: return obs_tma_coop_kernel<3, 2, 2, 32, true>;
-            case 3230204: return obs_tma_coop_kernel<3, 2, 4, 32, true>;
-            case 1630201: return obs_tma_coop_kernel<3, 2, 1, 16, true>;
-            case 1630202: return obs_tma_coop_kernel<3, 2, 2, 16, true>;
-            case 1630204: return obs_tma_coop_kernel<3, 2, 4, 16, true>;
-            case 830201: return obs_tma_coop_kernel<3, 2, 1, 8, true>;
-            case 830202: return obs_tma_coop_kernel<3, 2, 2, 8, true>;
-            case 830204: return obs_tma_coop_kernel<3, 2, 4, 8, true>;
-            default: return nullptr;
-        }
-    }
-    if (unit == 16) {
-        switch (key) {
-            case 30201: return obs_tma_coop_kernel<3, 2, 1, 16>;
-            case 30202: return obs_tma_coop_kernel<3, 2, 2, 16>;
-            case 30204: return obs_tma_coop_kernel<3, 2, 4, 16>;
-            default: return nullptr;
-        }
-    }
-    if (unit == 8) {
-        switch (key) {
-            case 30201: return obs_tma_coop_kernel<3, 2, 1, 8>;
-            case 30202: return obs_tma_coop_kernel<3, 2, 2, 8>;
-            case 30204: return obs_tma_coop_kernel<3, 2, 4, 8>;
-            default: return nullptr;
-        }
-    }
-    switch (key) {
-        case 30201: return obs_tma_coop_kernel<3, 2, 1>;
-        case 30202: return obs_tma_coop_kernel<3, 2, 2>;
-        case 30204: return obs_tma_coop_kernel<3, 2, 4>;
-        case 30208: return obs_tma_coop_kernel<3, 2, 8>;
-        case 30304: return obs_tma_coop_kernel<3, 3, 4>;
-        case 40204: return obs_tma_coop_kernel<4, 2, 4>;
-        case 40304: return obs_tma_coop_kernel<4, 3, 4>;
-        case 20204: return obs_tma_coop_kernel<2, 2, 4>;
-        case 40202: return obs_tma_coop_kernel<4, 2, 2>;
-        case 60202: return obs_tma_coop_kernel<6, 2, 2>;
-        case 60302: return obs_tma_coop_kernel<6, 3, 2>;
-        case 20208: return obs_tma_coop_kernel<2, 2, 8>;
-        default: return nullptr;
-    }
+    return gen ? tma_kernel_of<true>(key, unit, fused, dyn) : tma_kernel_of<false>(key, unit, fused, dyn);
 }
 
 // Pipeline shape: 3 window stages of the largest group (4, 2, 1 envs) + 2 ring tiles that still leave two CTAs per
@@ -640,6 +572,21 @@ static TmaConfig tma_config(const ObsShape& sh) {
 }
 
 // ------------------------------------------------------------------------------------------ launch
+using GenericKernelFn = void (*)(const GteParams, const GteData, const GteState, float*, const ObsShape, int, int);
+
+// the generic gather with G lanes per env
+template <bool GEN>
+static GenericKernelFn generic_kernel(int G) {
+    switch (G) {
+        case 32: return obs_generic_kernel<32, GEN>;
+        case 16: return obs_generic_kernel<16, GEN>;
+        case 8: return obs_generic_kernel<8, GEN>;
+        case 4: return obs_generic_kernel<4, GEN>;
+        case 2: return obs_generic_kernel<2, GEN>;
+        default: return obs_generic_kernel<1, GEN>;
+    }
+}
+
 bool obs_vec_supported(const GteParams& P, const GteData& D) {
     const ObsShape sh = make_shape(P);
     if (P.windows <= 0 || sh.win_bytes % 16 != 0) return false;
@@ -812,25 +759,8 @@ cudaError_t launch_obs_range(const GteParams& P, const GteData& D, const GteStat
         while (G > 1 && G / 2 >= per_env) G /= 2;
         const int64_t need = ((int64_t)n_envs * G + 255) / 256;
         const int grid = (int)(need < (int64_t)sms * 16 ? need : (int64_t)sms * 16);
-        if (sh.dyn.general) {
-            switch (G) {
-                case 32: obs_generic_kernel<32, true><<<grid, 256, 0, stream>>>(P, D, S, obs, sh, env_begin, env_end); break;
-                case 16: obs_generic_kernel<16, true><<<grid, 256, 0, stream>>>(P, D, S, obs, sh, env_begin, env_end); break;
-                case 8: obs_generic_kernel<8, true><<<grid, 256, 0, stream>>>(P, D, S, obs, sh, env_begin, env_end); break;
-                case 4: obs_generic_kernel<4, true><<<grid, 256, 0, stream>>>(P, D, S, obs, sh, env_begin, env_end); break;
-                case 2: obs_generic_kernel<2, true><<<grid, 256, 0, stream>>>(P, D, S, obs, sh, env_begin, env_end); break;
-                default: obs_generic_kernel<1, true><<<grid, 256, 0, stream>>>(P, D, S, obs, sh, env_begin, env_end); break;
-            }
-            return cudaGetLastError();
-        }
-        switch (G) {
-            case 32: obs_generic_kernel<32><<<grid, 256, 0, stream>>>(P, D, S, obs, sh, env_begin, env_end); break;
-            case 16: obs_generic_kernel<16><<<grid, 256, 0, stream>>>(P, D, S, obs, sh, env_begin, env_end); break;
-            case 8: obs_generic_kernel<8><<<grid, 256, 0, stream>>>(P, D, S, obs, sh, env_begin, env_end); break;
-            case 4: obs_generic_kernel<4><<<grid, 256, 0, stream>>>(P, D, S, obs, sh, env_begin, env_end); break;
-            case 2: obs_generic_kernel<2><<<grid, 256, 0, stream>>>(P, D, S, obs, sh, env_begin, env_end); break;
-            default: obs_generic_kernel<1><<<grid, 256, 0, stream>>>(P, D, S, obs, sh, env_begin, env_end); break;
-        }
+        const GenericKernelFn kern = sh.dyn.general ? generic_kernel<true>(G) : generic_kernel<false>(G);
+        kern<<<grid, 256, 0, stream>>>(P, D, S, obs, sh, env_begin, env_end);
         return cudaGetLastError();
     }
     if (variant == GTE_OBS_VEC) {

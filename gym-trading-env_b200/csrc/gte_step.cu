@@ -17,7 +17,8 @@ namespace gte {
 
 // Each CTA owns `tiles_per_cta` CONSECUTIVE 256-env tiles: 1 while the grid fits on the GPU at once, more beyond that
 // (see step_tiles_per_cta).  GEN: the general dynamic-feature catalogue (K0.dyn); every kernel below that writes the
-// ring has such an instantiation beside the one for no dynamic columns / the default pair.
+// ring runs one code path, instantiated with GEN = false for no dynamic columns / the default pair, whose ring layout
+// is then known at compile time (RingLayout).
 template <int MIN_CTAS, bool GEN = false>
 __global__ void __launch_bounds__(kStepThreads, MIN_CTAS)
 step_kernel(const GteParams P, const GteData D, const GteState S, const void* __restrict__ actions, const StepConsts K0,
@@ -45,7 +46,7 @@ step_kernel(const GteParams P, const GteData D, const GteState S, const void* __
         if (valid) r = step_env_now<GEN>(P, D, S, actions, K, O, tick, ring_slot, autoreset, (int)i, acc, s_pos);
         // windows=None (environments.py:156-157): the observation is the single row idx, written by the step kernel
         // itself -> one launch per lockstep iteration at small N
-        if (obs_rows != nullptr) write_obs_rows<GEN>(P, D, obs_rows, i, valid, r, obs_on_host != 0);
+        if (obs_rows != nullptr) write_obs_rows<GEN>(P, D, K.dyn, obs_rows, i, valid, r, obs_on_host != 0);
     }
     reduce_metrics<kStepThreads>(acc, O, S, chunk_flags);
 }
@@ -96,7 +97,7 @@ rollout_kernel(const GteParams P, const GteData D, const GteState S, const void*
             const StepThreadOut r = step_env<false, GEN>(P, D, S, K, o, tick0 + (uint64_t)k, ring_slot_of(P, clock0 + 1ull + (uint64_t)k),
                                                          autoreset, (int)i, in, p0, p1, acc, s_pos, &e);
             if (obs_rows != nullptr && (keep_obs || k == n_steps - 1))
-                write_obs_rows<GEN>(P, D, obs_rows + (keep_obs ? (int64_t)k * N * F : 0), i, true, r, false);
+                write_obs_rows<GEN>(P, D, K.dyn, obs_rows + (keep_obs ? (int64_t)k * N * F : 0), i, true, r, false);
         }
     }
     if (valid) store_env(S, i, e);
@@ -208,7 +209,7 @@ serve_kernel(const GteParams P, const GteData D, const GteState S, const StepCon
             load_prices(P, D, in, p0, p1);
             r = step_env<true, GEN>(P, D, S, K, O, tick, ring_slot, autoreset, (int)i, in, p0, p1, acc, s_pos);
         }
-        if (obs_rows != nullptr) write_obs_rows<GEN>(P, D, obs_rows, i, valid, r, obs_on_host != 0);
+        if (obs_rows != nullptr) write_obs_rows<GEN>(P, D, K.dyn, obs_rows, i, valid, r, obs_on_host != 0);
         GteStepOut o = O;
         o.seq_value = seq;                               // what the last CTA publishes to the host when all is visible
         reduce_metrics<kStepThreads>(acc, o, S, kChunkFirst | kChunkLast);

@@ -11,7 +11,7 @@ constexpr int kChunkFirst = 1, kChunkLast = 2, kChunkTotalOnly = 4;
 struct StepThreadOut {       // what the gather phase of the fused kernel needs from the step phase
     int idx, ep_start, ds;   // post-reset row index, episode start, dataset
     float dyn_pos, dyn_rp;   // the dynamic features of row idx (position, real_position), as written to the ring
-    float dyn_pr, dyn_rew, dyn_prog;   // general catalogue only: portfolio_return, reward, episode_progress of row idx
+    float dyn_pr, dyn_rew, dyn_prog;   // portfolio_return, reward, episode_progress of row idx (read when configured)
 };
 
 struct MetricAcc {           // per-thread accumulators (deterministic: fixed tile order per thread)
@@ -187,19 +187,17 @@ __device__ __forceinline__ StepThreadOut step_env(const GteParams& P, const GteD
         O.pre_reset_portfolio[2 * N + i] = e.pf.ia;
         O.pre_reset_portfolio[3 * N + i] = e.pf.ifi;
     }
+    const RingLayout<GEN> R{K.dyn};
     float dyn_pos = (float)pos_tab[e.pos_idx], dyn_rp = (float)rp;        // fp64 -> fp32 as numpy casts (:154)
-    float dyn_pr = 0.0f, dyn_rew = 0.0f, dyn_prog = 0.0f;
+    float dyn_pr = 0.0f, dyn_rew = (float)rew, dyn_prog = 0.0f;
+    // each value only when its kind is configured (the transition is issue-bound on fp64 divides)
+    if (R.kind_block(GTE_DYN_PORTFOLIO_RETURN) != kDynNone) dyn_pr = (float)dsub(ddiv(val, P.v0), 1.0);
+    if (R.kind_block(GTE_DYN_EPISODE_PROGRESS) != kDynNone)
+        dyn_prog = (float)ddiv((double)e.step, (double)P.max_episode_duration);
     // _get_obs write-back (:153-154); an auto-reset below overwrites the same slot with the new episode's first row
-    if (GEN) {
-        // each value only when its kind is configured (the transition is issue-bound on fp64 divides)
-        if (dyn_block_of(K.dyn, GTE_DYN_PORTFOLIO_RETURN) != kDynNone) dyn_pr = (float)dsub(ddiv(val, P.v0), 1.0);
-        dyn_rew = (float)rew;
-        if (dyn_block_of(K.dyn, GTE_DYN_EPISODE_PROGRESS) != kDynNone)
-            dyn_prog = (float)ddiv((double)e.step, (double)P.max_episode_duration);
+    if (P.n_dyn > 0) {
         const DynRow row = {dyn_rp, dyn_pr, dyn_rew, dyn_prog, e.pos_idx};
-        ring_store_dyn(P, K.dyn, S, i, ring_slot, row);
-    } else if (P.n_dyn > 0) {
-        ring_store(P, S, i, ring_slot, dyn_rp, e.pos_idx);
+        ring_store<GEN>(P, K.dyn, S, i, ring_slot, row);
     }
     acc.sum_rew = dadd(acc.sum_rew, rew);
     if (done || trunc) {                                                     // :269-271 calculate_metrics
@@ -238,6 +236,15 @@ __device__ __forceinline__ StepThreadOut step_env_now(const GteParams& P, const 
     return step_env<true, GEN>(P, D, S, K, O, tick, ring_slot, autoreset, i, in, p0, p1, acc, pos_tab);
 }
 
+// Dynamic column j of r: the value of the kind whose ring block column j reads.
+template <bool GEN>
+__device__ __forceinline__ float dyn_value(const RingLayout<GEN>& R, const StepThreadOut& r, int j) {
+    if (R.is_pos(j)) return r.dyn_pos;
+    const uint32_t b = (uint32_t)R.f32_block(j);
+    return b == R.kind_block(GTE_DYN_REAL_POSITION) ? r.dyn_rp : b == R.kind_block(GTE_DYN_PORTFOLIO_RETURN) ? r.dyn_pr
+         : b == R.kind_block(GTE_DYN_REWARD) ? r.dyn_rew : r.dyn_prog;
+}
+
 // The one-row observations (windows=None, environments.py:156-157) of the 32 consecutive envs of a warp; every lane of
 // the warp must call it (valid = this lane's env exists and r holds its step's result).
 //   coalesced = false: each lane writes its own row — 4-byte stores 4*F bytes apart; fine for device memory, where L2
@@ -246,25 +253,20 @@ __device__ __forceinline__ StepThreadOut step_env_now(const GteParams& P, const 
 //                      fetching (row, dataset, dynamic features) of the owning env by shuffle -> full 128-byte stores.
 //                      For MAPPED HOST memory, where every partial-sector store is its own PCIe transaction
 //                      (4096 envs: 60 us -> 27 us per host step).
-// GEN: dynamic columns in P.dyn_kinds order (general catalogue), else the default pair.
-__device__ __forceinline__ float dyn_value(const StepThreadOut& r, uint32_t kind) {
-    return kind == GTE_DYN_POSITION ? r.dyn_pos : kind == GTE_DYN_REAL_POSITION ? r.dyn_rp
-         : kind == GTE_DYN_PORTFOLIO_RETURN ? r.dyn_pr : kind == GTE_DYN_REWARD ? r.dyn_rew : r.dyn_prog;
-}
+// GEN: dynamic columns in P.dyn_kinds order (general catalogue), else the default pair (RingLayout).
 template <bool GEN = false>
-__device__ __forceinline__ void write_obs_rows(const GteParams& P, const GteData& D, float* __restrict__ obs_rows, int64_t i,
-                                               bool valid, const StepThreadOut& r, bool coalesced) {
+__device__ __forceinline__ void write_obs_rows(const GteParams& P, const GteData& D, const DynLayout& L,
+                                               float* __restrict__ obs_rows, int64_t i, bool valid, const StepThreadOut& r,
+                                               bool coalesced) {
+    const RingLayout<GEN> R{L};
     const int F = P.n_static + P.n_dyn;
     if (!coalesced) {
         if (valid) {
             const float* __restrict__ f = D.features + ((int64_t)r.ds * P.t_stride + r.idx) * P.n_static;
             float* __restrict__ o = obs_rows + i * F;
             for (int c = 0; c < P.n_static; ++c) o[c] = __ldg(f + c);
-            if (GEN) {
-                for (int j = 0; j < P.n_dyn; ++j) o[P.n_static + j] = dyn_value(r, ((uint32_t)P.dyn_kinds >> (4 * j)) & 15u);
-            } else if (P.n_dyn > 0) {
-                o[P.n_static] = r.dyn_pos; o[P.n_static + 1] = r.dyn_rp;
-            }
+            if (P.n_dyn > 0)
+                for (int j = 0; j < R.n_cols(); ++j) o[P.n_static + j] = dyn_value(R, r, j);
         }
         return;
     }
@@ -274,20 +276,15 @@ __device__ __forceinline__ void write_obs_rows(const GteParams& P, const GteData
     for (int j = lane; j < 32 * F; j += 32) {                    // F trips for every lane
         const int e = j / F, c = j - e * F;
         const int idx = __shfl_sync(FULL, r.idx, e), ds = __shfl_sync(FULL, r.ds, e);
-        const float dp = __shfl_sync(FULL, r.dyn_pos, e), dr = __shfl_sync(FULL, r.dyn_rp, e);
+        StepThreadOut q;
+        q.dyn_pos = __shfl_sync(FULL, r.dyn_pos, e);
+        q.dyn_rp = __shfl_sync(FULL, r.dyn_rp, e);
+        q.dyn_pr = __shfl_sync(FULL, r.dyn_pr, e);
+        q.dyn_rew = __shfl_sync(FULL, r.dyn_rew, e);
+        q.dyn_prog = __shfl_sync(FULL, r.dyn_prog, e);
         const bool ok = __shfl_sync(FULL, (int)valid, e) != 0;
-        if (GEN) {
-            StepThreadOut q;
-            q.dyn_pos = dp; q.dyn_rp = dr;
-            q.dyn_pr = __shfl_sync(FULL, r.dyn_pr, e);
-            q.dyn_rew = __shfl_sync(FULL, r.dyn_rew, e);
-            q.dyn_prog = __shfl_sync(FULL, r.dyn_prog, e);
-            if (ok) o[j] = c < P.n_static ? __ldg(D.features + ((int64_t)ds * P.t_stride + idx) * P.n_static + c)
-                                          : dyn_value(q, ((uint32_t)P.dyn_kinds >> (4 * (c - P.n_static))) & 15u);
-        } else {
-            if (ok) o[j] = c < P.n_static ? __ldg(D.features + ((int64_t)ds * P.t_stride + idx) * P.n_static + c)
-                                          : (c == P.n_static ? dp : dr);
-        }
+        if (ok) o[j] = c < P.n_static ? __ldg(D.features + ((int64_t)ds * P.t_stride + idx) * P.n_static + c)
+                                      : dyn_value(R, q, c - P.n_static);
     }
 }
 

@@ -35,20 +35,20 @@ extern "C" {
 #define GTE_MAX_POSITIONS 64
 #define GTE_MAX_DATASETS 64        /* least-used rotation keeps a 64-bit "used this round" mask per env */
 #define GTE_N_METRICS 8
-/* dynamic-feature ring: one block per tile of 32 consecutive envs (layout at GteState.dyn_ring) */
+/* dynamic-feature ring: one block per tile of 32 consecutive envs (layout at GteState.dyn_ring) for any dynamic-feature
+ * catalogue (GteParams.dyn_kinds): n_f32 blocks of W rows x 32 f32 values, one per f32 kind, then n_pos (0 or 1) blocks
+ * of W rows x 32 u8 position indices. */
 #define GTE_RING_TILE_ENVS 32
-#define GTE_RING_TILE_BYTES(W) ((W) * 160)
-#define GTE_RING_BYTES(N, W) ((((int64_t)(N) + 31) / 32) * GTE_RING_TILE_BYTES(W))
-#define GTE_RING_RP_OFFSET(s, e) ((s) * 128 + (((((e) >> 2) ^ ((s) & 7))) << 4) + (((e) & 3) << 2))
-#define GTE_RING_POS_OFFSET(W, s, e) ((W) * 128 + (s) * 32 + (e))
-/* The same layout for any dynamic-feature catalogue (GteParams.dyn_kinds): n_f32 blocks of W rows x 32 f32 values, one
- * per f32 kind, then n_pos (0 or 1) blocks of W rows x 32 u8 position indices.  With n_f32 = n_pos = 1 these are byte
- * for byte GTE_RING_TILE_BYTES / GTE_RING_RP_OFFSET / GTE_RING_POS_OFFSET. */
 #define GTE_MAX_DYN 5
 #define GTE_RING_TILE_BYTES_DYN(W, n_f32, n_pos) ((W) * (128 * (n_f32) + 32 * (n_pos)))
 #define GTE_RING_BYTES_DYN(N, W, n_f32, n_pos) ((((int64_t)(N) + 31) / 32) * GTE_RING_TILE_BYTES_DYN(W, n_f32, n_pos))
-#define GTE_RING_F32_OFFSET(W, k, s, e) ((k) * (W) * 128 + GTE_RING_RP_OFFSET(s, e))
+#define GTE_RING_F32_OFFSET(W, k, s, e) ((k) * (W) * 128 + (s) * 128 + (((((e) >> 2) ^ ((s) & 7))) << 4) + (((e) & 3) << 2))
 #define GTE_RING_POS_OFFSET_DYN(W, n_f32, s, e) ((n_f32) * (W) * 128 + (s) * 32 + (e))
+/* The default pair (position, real_position): n_f32 = n_pos = 1, real_position in f32 block 0. */
+#define GTE_RING_TILE_BYTES(W) GTE_RING_TILE_BYTES_DYN(W, 1, 1)
+#define GTE_RING_BYTES(N, W) GTE_RING_BYTES_DYN(N, W, 1, 1)
+#define GTE_RING_RP_OFFSET(s, e) GTE_RING_F32_OFFSET(0, 0, s, e)
+#define GTE_RING_POS_OFFSET(W, s, e) GTE_RING_POS_OFFSET_DYN(W, 1, s, e)
 #define GTE_STEP_THREADS 256       /* envs per tile of the step kernel */
 #define GTE_MAX_PARTIAL_ROWS 4096  /* rows of GteStepOut.metric_partials (one per CTA; every grid is capped at this) */
 /* Result block of gte_step_host — everything a host policy needs back from one iteration, in ONE piece of memory
