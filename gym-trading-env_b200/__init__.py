@@ -19,12 +19,17 @@ _LAZY = {"TradingVectorEnv", "MultiDatasetTradingVectorEnv", "basic_reward_funct
          "DeviceReward", "log_return_reward", "simple_return_reward"}
 _FEATURES = {"DeviceFeature", "parse_dynamic_features", "portfolio_return_feature", "reward_feature",
              "episode_progress_feature"}
+_METRICS = {"DeviceMetric", "position_changes_metric", "episode_length_metric", "max_drawdown_metric",
+            "episode_reward_metric", "time_in_market_metric"}
 
 
 def __getattr__(name):          # torch / the CUDA library are only imported when an env class is used
     if name in _FEATURES:             # host-only: importable without torch or a device
         from . import dynamic_features
         return getattr(dynamic_features, name)
+    if name in _METRICS:              # host-only as well
+        from . import episode_metrics
+        return getattr(episode_metrics, name)
     if name in _LAZY:
         from . import vector_env
         return getattr(vector_env, name)

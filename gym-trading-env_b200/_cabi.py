@@ -25,6 +25,11 @@ GTE_N_METRICS = 8
 GTE_STEP_THREADS = 256
 GTE_MAX_PARTIAL_ROWS = 4096
 GTE_MAX_DYN = 5
+GTE_N_METRIC_KINDS = 5            # enum GteMetricKind: metric_kinds bit 1 << kind
+GTE_METRIC_KINDS_ALL = 0x1f
+GTE_METRIC_KINDS_STATEFUL = 0x1d  # every kind but episode_length keeps state in episode_acc
+GTE_EPISODE_ACC_ROWS = 5
+GTE_EPISODE_RECORD_ROWS = 7
 
 
 def ring_tile_bytes(windows: int, n_dyn: int, dyn_kinds: int) -> int:
@@ -53,6 +58,7 @@ class GteParams(C.Structure):
         ("fee", C.c_double), ("rate", C.c_double), ("v0", C.c_double), ("done_ratio", C.c_double),
         ("reward_scale", C.c_double), ("reward_lo", C.c_double), ("reward_hi", C.c_double),
         ("positions", C.c_double * GTE_MAX_POSITIONS),
+        ("metric_kinds", C.c_int32), ("pad_metric", C.c_int32),
     ]
 
 
@@ -72,7 +78,7 @@ class GteState(C.Structure):
         ("dyn_ring", C.c_void_p), ("ring_clock", C.c_void_p),
         ("plan_cursor", C.c_void_p), ("ds_used", C.c_void_p), ("ds_episodes", C.c_void_p),
         ("reset_plan", C.c_void_p), ("limit_price", C.c_void_p), ("limit_seq", C.c_void_p),
-        ("error_flag", C.c_void_p), ("tick", C.c_void_p),
+        ("error_flag", C.c_void_p), ("tick", C.c_void_p), ("episode_acc", C.c_void_p),
     ]
 
 
@@ -85,7 +91,7 @@ class GteStepOut(C.Structure):
         ("metrics_total", C.c_void_p), ("block_counter", C.c_void_p), ("error_out", C.c_void_p),
         ("seq_out", C.c_void_p), ("seq_value", C.c_uint32), ("ended_cap", C.c_uint32),
         ("ended_list", C.c_void_p), ("ended_counter", C.c_void_p), ("ended_n_out", C.c_void_p),
-        ("reward_f32", C.c_void_p),
+        ("reward_f32", C.c_void_p), ("episode_record", C.c_void_p),
     ]
 
 

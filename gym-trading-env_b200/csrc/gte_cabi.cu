@@ -42,6 +42,14 @@ const char* bad_dyn_kinds(const GteParams* p) {
     return nullptr;
 }
 
+// GteParams.metric_kinds: known kind bits only; the stateful kinds need GteState.episode_acc
+const char* bad_metric_kinds(const GteParams* p, const GteState* s) {
+    if ((p->metric_kinds & ~GTE_METRIC_KINDS_ALL) != 0) return "metric_kinds: a bit outside GTE_METRIC_KINDS_ALL";
+    if ((p->metric_kinds & GTE_METRIC_KINDS_STATEFUL) != 0 && s->episode_acc == nullptr)
+        return "metric_kinds: the configured kinds need episode_acc";
+    return nullptr;
+}
+
 int check_common(const char* fn, const GteParams* p, const GteData* d, const GteState* s) {
     GTE_REQUIRE(fn, p != nullptr && d != nullptr && s != nullptr);
     GTE_REQUIRE(fn, p->n_envs > 0);
@@ -65,6 +73,7 @@ int check_common(const char* fn, const GteParams* p, const GteData* d, const Gte
     GTE_REQUIRE(fn, p->n_dyn == 0 || (s->dyn_ring != nullptr && (reinterpret_cast<uintptr_t>(s->dyn_ring) & 15u) == 0));
     GTE_REQUIRE(fn, s->plan_cursor && s->ds_used && s->ds_episodes && s->error_flag && s->tick);
     GTE_REQUIRE(fn, p->plan_episodes == 0 || s->reset_plan != nullptr);
+    if (const char* why = bad_metric_kinds(p, s)) return fail_arg(fn, why);
     GTE_REQUIRE(fn, p->n_limit_positions >= 0 && p->n_limit_positions <= p->n_positions);
     GTE_REQUIRE(fn, p->n_limit_positions == 0 || (s->limit_price && s->limit_seq && d->high && d->low));
     GTE_REQUIRE(fn, p->action_bytes == 0 || p->action_bytes == 1 || p->action_bytes == 2 || p->action_bytes == 4 || p->action_bytes == 8);
@@ -97,8 +106,11 @@ int gte_reset(const GteParams* params, const GteData* data, const GteState* stat
                                                      static_cast<cudaStream_t>(stream)));
 }
 
-static int check_step_out(const char* fn, const void* actions, const GteStepOut* out, bool own_results = false) {
+static int check_step_out(const char* fn, const GteParams* params, const void* actions, const GteStepOut* out,
+                          bool own_results = false) {
     GTE_REQUIRE(fn, actions != nullptr && out != nullptr);
+    if (params->metric_kinds != 0 && out->episode_record == nullptr)
+        return fail_arg(fn, "metric_kinds: episode metrics need episode_record");
     GTE_REQUIRE(fn, own_results || (out->reward && out->terminated && out->truncated));
     GTE_REQUIRE(fn, out->metric_partials && out->metrics_step && out->block_counter);
     return GTE_OK;
@@ -118,7 +130,7 @@ static int check_obs_ptr(const char* fn, const GteParams* params, const GteData*
 int gte_step(const GteParams* params, const GteData* data, const GteState* state, const void* actions,
              const GteStepOut* out, int autoreset, void* stream) {
     if (int rc = check_common("gte_step", params, data, state)) return rc;
-    if (int rc = check_step_out("gte_step", actions, out)) return rc;
+    if (int rc = check_step_out("gte_step", params, actions, out)) return rc;
     return check_cuda("gte_step", gte::launch_step(*params, *data, *state, actions, *out, autoreset,
                                                    static_cast<cudaStream_t>(stream)));
 }
@@ -135,7 +147,7 @@ static int check_variant(const char* fn, const GteParams* params, const GteData*
 int gte_step_obs(const GteParams* params, const GteData* data, const GteState* state, const void* actions,
                  const GteStepOut* out, float* obs, int autoreset, int variant, int n_chunks, void* stream) {
     if (int rc = check_common("gte_step_obs", params, data, state)) return rc;
-    if (int rc = check_step_out("gte_step_obs", actions, out)) return rc;
+    if (int rc = check_step_out("gte_step_obs", params, actions, out)) return rc;
     GTE_REQUIRE("gte_step_obs", obs != nullptr && n_chunks >= 0 && n_chunks <= 16);
     if (int rc = check_variant("gte_step_obs", params, data, variant)) return rc;
     if (int rc = check_obs_ptr("gte_step_obs", params, data, obs, variant)) return rc;
@@ -147,7 +159,7 @@ int gte_step_host(const GteParams* params, const GteData* data, const GteState* 
                   const GteStepOut* out, float* obs, int autoreset, int variant, int* mode_used, void* stream) {
     if (int rc = check_common("gte_step_host", params, data, state)) return rc;
     GTE_REQUIRE("gte_step_host", io != nullptr && io->actions != nullptr && io->results != nullptr);
-    if (int rc = check_step_out("gte_step_host", io->actions, out, true)) return rc;
+    if (int rc = check_step_out("gte_step_host", params, io->actions, out, true)) return rc;
     GTE_REQUIRE("gte_step_host", io->mode >= GTE_IO_AUTO && io->mode <= GTE_IO_SERVER);
     GTE_REQUIRE("gte_step_host", (reinterpret_cast<uintptr_t>(io->results) & 7u) == 0);
     GTE_REQUIRE("gte_step_host", out->seq_out == nullptr);   // the call points it into the result block itself
@@ -165,7 +177,7 @@ int gte_step_host_begin(const GteParams* params, const GteData* data, const GteS
                         const GteStepOut* out, float* obs, int autoreset, int variant, void* stream) {
     if (int rc = check_common("gte_step_host_begin", params, data, state)) return rc;
     GTE_REQUIRE("gte_step_host_begin", io != nullptr && io->actions != nullptr && io->results != nullptr);
-    if (int rc = check_step_out("gte_step_host_begin", io->actions, out, true)) return rc;
+    if (int rc = check_step_out("gte_step_host_begin", params, io->actions, out, true)) return rc;
     GTE_REQUIRE("gte_step_host_begin", io->dev_actions != nullptr && io->dev_results != nullptr);
     GTE_REQUIRE("gte_step_host_begin", ((reinterpret_cast<uintptr_t>(io->results) | reinterpret_cast<uintptr_t>(io->dev_results)) & 7u) == 0);
     GTE_REQUIRE("gte_step_host_begin", io->obs_host == nullptr && out->seq_out == nullptr);
@@ -229,7 +241,7 @@ int gte_host_unregister(void* ptr) {
 int gte_rollout(const GteParams* params, const GteData* data, const GteState* state, const void* actions,
                 int n_steps, const GteStepOut* out, float* obs, int keep_obs, int autoreset, int variant, void* stream) {
     if (int rc = check_common("gte_rollout", params, data, state)) return rc;
-    if (int rc = check_step_out("gte_rollout", actions, out)) return rc;
+    if (int rc = check_step_out("gte_rollout", params, actions, out)) return rc;
     GTE_REQUIRE("gte_rollout", obs != nullptr && n_steps >= 1);
     if (int rc = check_variant("gte_rollout", params, data, variant)) return rc;
     if (int rc = check_obs_ptr("gte_rollout", params, data, obs, variant)) return rc;
@@ -270,6 +282,7 @@ int gte_struct_size(int which) {
 int gte_step_obs_launches(const GteParams* params, const GteData* data, int variant, int n_chunks) {
     if (params == nullptr || data == nullptr || n_chunks < 0 || n_chunks > 16) return GTE_ERR_ARG;
     if (params->windows == 0) return 1;
+    // (episode metrics: the fused form is never taken, step_obs_is_fused says so)
     if (n_chunks == 0 && gte::default_chunks(params->n_envs) == 1 && gte::step_obs_is_fused(*params, *data, variant)) return 1;
     return 2 * (n_chunks == 0 ? gte::default_chunks(params->n_envs) : n_chunks);
 }

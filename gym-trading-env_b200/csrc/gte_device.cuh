@@ -255,10 +255,28 @@ struct EnvRegs {          // the per-env state a step keeps in registers
     int pos_idx, step, ep_start, ds;
 };
 
+// Episode metrics (GteParams.metric_kinds, TradingEnv.add_metric :274-294): the running state of env i's episode in
+// GteState.episode_acc, one f64 row per quantity (enum GteEpisodeAccRow).  Only the rows of configured kinds are touched.
+__device__ __forceinline__ bool metric_on(const GteParams& P, int kind) { return (P.metric_kinds >> kind) & 1; }
+
+// The reset row (:186-197): valuation v0, reward 0, the episode's first position.
+__device__ __forceinline__ void episode_acc_init(const GteParams& P, const GteState& S, int i, double position) {
+    const int64_t N = P.n_envs;
+    double* __restrict__ A = S.episode_acc;
+    if (metric_on(P, GTE_METRIC_MAX_DRAWDOWN)) {
+        A[GTE_ACC_PEAK * N + i] = P.v0;
+        A[GTE_ACC_DRAWDOWN * N + i] = 0.0;                                    // 1 - v0 / v0
+    }
+    if (metric_on(P, GTE_METRIC_EPISODE_REWARD)) A[GTE_ACC_REWARD_SUM * N + i] = 0.0;
+    if (metric_on(P, GTE_METRIC_POSITION_CHANGES)) A[GTE_ACC_POSITION_CHANGES * N + i] = 0.0;
+    if (metric_on(P, GTE_METRIC_TIME_IN_MARKET)) A[GTE_ACC_IN_MARKET * N + i] = (position != 0.0) ? 1.0 : 0.0;
+}
+
 // TradingEnv.reset (environments.py:163-199) preceded by MultiDatasetTradingEnv.reset (:393-400).
 // Rare path (once per episode): plan/rotation bookkeeping goes straight to global memory.
 // GEN: the general dynamic-feature catalogue (L.general), else no dynamic columns or the default pair (RingLayout).
-template <bool GEN = false>
+// ACC: episode metrics are configured (metric_kinds != 0): the episode's accumulators start from the reset row.
+template <bool GEN = false, bool ACC = false>
 __device__ __forceinline__ void reset_env(const GteParams& P, const GteData& D, const GteState& S,
                                        int i, uint64_t tick, int ring_slot, EnvRegs& e, const DynLayout& L) {
     uint32_t r[4];
@@ -313,6 +331,7 @@ __device__ __forceinline__ void reset_env(const GteParams& P, const GteData& D, 
         const DynRow r = {(float)position, 0.0f, 0.0f, 0.0f, e.pos_idx};
         ring_store<GEN>(P, L, S, i, ring_slot, r);
     }
+    if (ACC) episode_acc_init(P, S, i, position);
 }
 
 }  // namespace gte

@@ -18,8 +18,9 @@ namespace gte {
 // Each CTA owns `tiles_per_cta` CONSECUTIVE 256-env tiles: 1 while the grid fits on the GPU at once, more beyond that
 // (see step_tiles_per_cta).  GEN: the general dynamic-feature catalogue (K0.dyn); every kernel below that writes the
 // ring runs one code path, instantiated with GEN = false for no dynamic columns / the default pair, whose ring layout
-// is then known at compile time (RingLayout).
-template <int MIN_CTAS, bool GEN = false>
+// is then known at compile time (RingLayout).  ACC (here and in every kernel below): episode metrics are configured
+// (metric_kinds != 0); the ACC = false instantiations are the kernels of a run without them.
+template <int MIN_CTAS, bool GEN = false, bool ACC = false>
 __global__ void __launch_bounds__(kStepThreads, MIN_CTAS)
 step_kernel(const GteParams P, const GteData D, const GteState S, const void* __restrict__ actions, const StepConsts K0,
             const GteStepOut O, int autoreset, int tiles_per_cta, int env_begin, int env_end, int chunk_flags,
@@ -43,7 +44,7 @@ step_kernel(const GteParams P, const GteData D, const GteState S, const void* __
         const int64_t i = base0 + (int64_t)t * kStepThreads + threadIdx.x;
         const bool valid = i < env_end;
         StepThreadOut r = {};
-        if (valid) r = step_env_now<GEN>(P, D, S, actions, K, O, tick, ring_slot, autoreset, (int)i, acc, s_pos);
+        if (valid) r = step_env_now<GEN, ACC>(P, D, S, actions, K, O, tick, ring_slot, autoreset, (int)i, acc, s_pos);
         // windows=None (environments.py:156-157): the observation is the single row idx, written by the step kernel
         // itself -> one launch per lockstep iteration at small N
         if (obs_rows != nullptr) write_obs_rows<GEN>(P, D, K.dyn, obs_rows, i, valid, r, obs_on_host != 0);
@@ -58,7 +59,8 @@ step_kernel(const GteParams P, const GteData D, const GteState S, const void* __
 // then costs the transition's own dependency chain (~1.5 us) instead of a kernel launch (~8 us).
 // Every per-env output array of O holds n_steps consecutive copies, iteration k writing copy k (gte_rollout).
 // obs_rows (windows == 0 only): the one-row observations, every iteration (keep_obs) or the last one.
-template <bool GEN = false>
+// The episode record is not replicated: it ends up holding the last episode each env finished.
+template <bool GEN = false, bool ACC = false>
 __global__ void __launch_bounds__(kStepThreads, 2)
 rollout_kernel(const GteParams P, const GteData D, const GteState S, const void* __restrict__ actions, const StepConsts K0,
                const GteStepOut O, int autoreset, int n_steps, int keep_obs, float* __restrict__ obs_rows) {
@@ -94,7 +96,7 @@ rollout_kernel(const GteParams P, const GteData D, const GteState S, const void*
             if (o.info_idx) o.info_idx += (int64_t)k * N;
             if (o.info_step) o.info_step += (int64_t)k * N;
             if (o.pre_reset_portfolio) o.pre_reset_portfolio += (int64_t)k * 4 * N;
-            const StepThreadOut r = step_env<false, GEN>(P, D, S, K, o, tick0 + (uint64_t)k, ring_slot_of(P, clock0 + 1ull + (uint64_t)k),
+            const StepThreadOut r = step_env<false, GEN, ACC>(P, D, S, K, o, tick0 + (uint64_t)k, ring_slot_of(P, clock0 + 1ull + (uint64_t)k),
                                                          autoreset, (int)i, in, p0, p1, acc, s_pos, &e);
             if (obs_rows != nullptr && (keep_obs || k == n_steps - 1))
                 write_obs_rows<GEN>(P, D, K.dyn, obs_rows + (keep_obs ? (int64_t)k * N * F : 0), i, true, r, false);
@@ -151,7 +153,7 @@ __device__ __forceinline__ int64_t load_action_volatile(const void* actions, int
     }
 }
 
-template <bool GEN = false>
+template <bool GEN = false, bool ACC = false>
 __global__ void __launch_bounds__(kStepThreads, 2)
 serve_kernel(const GteParams P, const GteData D, const GteState S, const StepConsts K0, const GteStepOut O, int autoreset,
              float* __restrict__ obs_rows, int obs_on_host, ServeCtl* ctl, unsigned long long* dctl, uint32_t first_seq,
@@ -207,7 +209,7 @@ serve_kernel(const GteParams P, const GteData D, const GteState S, const StepCon
             const EnvIn in = make_env_in(P, D, S, K, load_env_regs<true>(P, S, i), a);
             double p0, p1;
             load_prices(P, D, in, p0, p1);
-            r = step_env<true, GEN>(P, D, S, K, O, tick, ring_slot, autoreset, (int)i, in, p0, p1, acc, s_pos);
+            r = step_env<true, GEN, ACC>(P, D, S, K, O, tick, ring_slot, autoreset, (int)i, in, p0, p1, acc, s_pos);
         }
         if (obs_rows != nullptr) write_obs_rows<GEN>(P, D, K.dyn, obs_rows, i, valid, r, obs_on_host != 0);
         GteStepOut o = O;
@@ -222,7 +224,7 @@ serve_kernel(const GteParams P, const GteData D, const GteState S, const StepCon
 
 // TradingEnv.reset for the masked envs (environments.py:163-199, :393-400); `first` also performs
 // the dataset draw of MultiDatasetTradingEnv.__init__ (:377-378).
-template <bool GEN = false>
+template <bool GEN = false, bool ACC = false>
 __global__ void __launch_bounds__(kStepThreads)
 reset_kernel(const GteParams P, const GteData D, const GteState S, const uint8_t* __restrict__ mask,
              int first, const DynLayout L) {
@@ -245,7 +247,7 @@ reset_kernel(const GteParams P, const GteData D, const GteState S, const uint8_t
     if (mask != nullptr && mask[i] == 0) return;
     EnvRegs e;
     e.ds = S.dataset_idx[i];
-    reset_env<GEN>(P, D, S, i, tick, ring_slot_of(P, *S.ring_clock), e, L);    // the row currently observed
+    reset_env<GEN, ACC>(P, D, S, i, tick, ring_slot_of(P, *S.ring_clock), e, L);    // the row currently observed
     S.asset[i] = e.pf.asset;
     S.fiat[i] = e.pf.fiat;
     S.interest_asset[i] = e.pf.ia;
@@ -369,12 +371,15 @@ cudaError_t launch_step_range(const GteParams& P, const GteData& D, const GteSta
     if (!carveout_set[dev & 15]) {
         cudaFuncSetAttribute(step_kernel<3>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
         cudaFuncSetAttribute(step_kernel<3, true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+        cudaFuncSetAttribute(step_kernel<3, false, true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+        cudaFuncSetAttribute(step_kernel<3, true, true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
         carveout_set[dev & 15] = true;
     }
     // ONE build: 3 CTAs per SM at 80 registers with no local-memory spills.  The 4-CTAs/SM build (64 registers, 18 STL /
     // 15 LDL) measures the same on the C5 shard (0.0925 vs 0.0930 ms): the kernel is bound by the issue rate of its
     // dependent fp64 chains, not by resident warps, loads or stores (profiles/r02_tuning.md has the diagnostic runs)
-    auto kern = K.dyn.general ? step_kernel<3, true> : step_kernel<3>;
+    auto kern = P.metric_kinds != 0 ? (K.dyn.general ? step_kernel<3, true, true> : step_kernel<3, false, true>)
+                                    : (K.dyn.general ? step_kernel<3, true> : step_kernel<3>);
     return launch_pdl(kern, dim3(grid), dim3(kStepThreads), 0, stream, P, D, S, actions, K, O, autoreset, tpc,
                       env_begin, env_end, chunk_flags, obs_rows, obs_on_host ? 1 : 0);
 }
@@ -388,8 +393,9 @@ cudaError_t launch_reset(const GteParams& P, const GteData& D, const GteState& S
                          int first, cudaStream_t stream) {
     const int grid = (P.n_envs + kStepThreads - 1) / kStepThreads;
     const DynLayout L = dyn_layout(P);
-    if (L.general) reset_kernel<true><<<grid, kStepThreads, 0, stream>>>(P, D, S, mask, first, L);
-    else reset_kernel<<<grid, kStepThreads, 0, stream>>>(P, D, S, mask, first, L);
+    auto kern = P.metric_kinds != 0 ? (L.general ? reset_kernel<true, true> : reset_kernel<false, true>)
+                                    : (L.general ? reset_kernel<true> : reset_kernel<false>);
+    kern<<<grid, kStepThreads, 0, stream>>>(P, D, S, mask, first, L);
     bump_tick_kernel<<<1, 1, 0, stream>>>(S.tick);
     return cudaGetLastError();
 }
@@ -483,7 +489,9 @@ cudaError_t launch_rollout(const GteParams& P, const GteData& D, const GteState&
     if (rollout_is_persistent(P, n_steps, keep_obs)) {
         const int grid = (int)((N + kStepThreads - 1) / kStepThreads);
         const StepConsts K = make_step_consts(P);
-        e = launch_pdl(K.dyn.general ? rollout_kernel<true> : rollout_kernel<false>, dim3(grid), dim3(kStepThreads), 0, stream,
+        auto kern = P.metric_kinds != 0 ? (K.dyn.general ? rollout_kernel<true, true> : rollout_kernel<false, true>)
+                                        : (K.dyn.general ? rollout_kernel<true> : rollout_kernel<false>);
+        e = launch_pdl(kern, dim3(grid), dim3(kStepThreads), 0, stream,
                        P, D, S, actions, K, O, autoreset, n_steps, keep_obs, P.windows == 0 ? obs : (float*)nullptr);
         if (e != cudaSuccess || P.windows == 0) return e;
         return launch_obs_range(P, D, S, obs, variant, 0, P.n_envs, stream);     // the last iteration's windows
@@ -682,7 +690,8 @@ cudaError_t launch_step_host(const GteParams& P, const GteData& D, const GteStat
         if (io.obs_host != nullptr) obs = static_cast<float*>(io.obs_host);   // windows == 0: rows written straight to the host
         const bool same = h->serving && memcmp(&h->sp, &p0, sizeof(p0)) == 0 && memcmp(&h->sd, &D, sizeof(D)) == 0 &&
                           memcmp(&h->ss, &S, sizeof(S)) == 0 && h->so.metrics_step == O.metrics_step &&
-                          h->so.reward == o.reward && h->sobs == obs && h->sauto == autoreset;
+                          h->so.reward == o.reward && h->so.episode_record == O.episode_record &&
+                          h->sobs == obs && h->sauto == autoreset;
         if (h->serving && !same && (e = serve_quiesce()) != cudaSuccess) return e;
         auto launch = [&]() -> cudaError_t {
             cudaError_t le;
@@ -693,7 +702,8 @@ cudaError_t launch_step_host(const GteParams& P, const GteData& D, const GteStat
             h->ctl->alive = 1u;
             const int grid = (int)((N + kStepThreads - 1) / kStepThreads);
             const StepConsts K = make_step_consts(p0);
-            auto kern = K.dyn.general ? serve_kernel<true> : serve_kernel<false>;
+            auto kern = p0.metric_kinds != 0 ? (K.dyn.general ? serve_kernel<true, true> : serve_kernel<false, true>)
+                                             : (K.dyn.general ? serve_kernel<true> : serve_kernel<false>);
             kern<<<grid, kStepThreads, 0, h->serve>>>(p0, D, S, K, o, autoreset, obs, io.obs_host != nullptr ? 1 : 0, h->ctl,
                                                       h->dctl, seq, serve_idle_ns());
             if ((le = cudaGetLastError()) != cudaSuccess) return le;

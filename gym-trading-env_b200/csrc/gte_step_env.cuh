@@ -111,9 +111,60 @@ __device__ __forceinline__ void load_prices(const GteParams& P, const GteData& D
     p1 = __ldg(price + in.idx + 1);
 }
 
+// Episode metrics (ACC): the accumulators of env i after this step's History row (position after the market trade and
+// the limit orders, valuation, reward) has been folded in, in the reference's operation order.  Stored back every step.
+struct EpisodeAcc {
+    double peak, drawdown, reward_sum, changes, in_market;
+};
+__device__ __forceinline__ EpisodeAcc episode_acc_fold(const GteParams& P, const GteState& S, int i, double pos_before,
+                                                       double pos_after, double val, double rew) {
+    const int64_t N = P.n_envs;
+    double* __restrict__ A = S.episode_acc;
+    EpisodeAcc a = {0.0, 0.0, 0.0, 0.0, 0.0};
+    if (metric_on(P, GTE_METRIC_MAX_DRAWDOWN)) {
+        a.peak = __ldcg(A + GTE_ACC_PEAK * N + i);
+        a.drawdown = __ldcg(A + GTE_ACC_DRAWDOWN * N + i);
+        a.peak = (val > a.peak) ? val : a.peak;                              // np.maximum.accumulate(v)
+        const double d = dsub(1.0, ddiv(val, a.peak));                       // 1 - v / peak
+        a.drawdown = (d > a.drawdown) ? d : a.drawdown;                      // np.max
+        A[GTE_ACC_PEAK * N + i] = a.peak;
+        A[GTE_ACC_DRAWDOWN * N + i] = a.drawdown;
+    }
+    if (metric_on(P, GTE_METRIC_EPISODE_REWARD)) {                           // sum(): left to right
+        a.reward_sum = dadd(__ldcg(A + GTE_ACC_REWARD_SUM * N + i), rew);
+        A[GTE_ACC_REWARD_SUM * N + i] = a.reward_sum;
+    }
+    if (metric_on(P, GTE_METRIC_POSITION_CHANGES)) {                         // np.diff(position) != 0: History rows
+        a.changes = __ldcg(A + GTE_ACC_POSITION_CHANGES * N + i) + ((pos_after != pos_before) ? 1.0 : 0.0);
+        A[GTE_ACC_POSITION_CHANGES * N + i] = a.changes;
+    }
+    if (metric_on(P, GTE_METRIC_TIME_IN_MARKET)) {
+        a.in_market = __ldcg(A + GTE_ACC_IN_MARKET * N + i) + ((pos_after != 0.0) ? 1.0 : 0.0);
+        A[GTE_ACC_IN_MARKET * N + i] = a.in_market;
+    }
+    return a;
+}
+
+// The episode of env i ended with this step: its metrics into GteStepOut.episode_record (rows: include/gte_b200.h).
+__device__ __forceinline__ void episode_record(const GteParams& P, const GteStepOut& O, int i, const EpisodeAcc& a,
+                                               double market_return, double portfolio_return, int step) {
+    const int64_t N = P.n_envs;
+    double* __restrict__ R = O.episode_record;
+    const double len = (double)step + 1.0;                                   // len(history): the reset row + step rows
+    R[i] = market_return;
+    R[N + i] = portfolio_return;
+    if (metric_on(P, GTE_METRIC_POSITION_CHANGES)) R[(2 + GTE_METRIC_POSITION_CHANGES) * N + i] = a.changes;
+    if (metric_on(P, GTE_METRIC_EPISODE_LENGTH)) R[(2 + GTE_METRIC_EPISODE_LENGTH) * N + i] = len;
+    if (metric_on(P, GTE_METRIC_MAX_DRAWDOWN)) R[(2 + GTE_METRIC_MAX_DRAWDOWN) * N + i] = a.drawdown;
+    if (metric_on(P, GTE_METRIC_EPISODE_REWARD)) R[(2 + GTE_METRIC_EPISODE_REWARD) * N + i] = a.reward_sum;
+    if (metric_on(P, GTE_METRIC_TIME_IN_MARKET)) R[(2 + GTE_METRIC_TIME_IN_MARKET) * N + i] = ddiv(a.in_market, len);
+}
+
 // The arithmetic of one transition.  STORE_STATE = false: the caller keeps the env's state in registers across iterations
 // (rollout / server kernels) and takes it back through e_out.  GEN: the general dynamic-feature catalogue (K.dyn).
-template <bool STORE_STATE = true, bool GEN = false>
+// ACC: episode metrics are configured (P.metric_kinds != 0): every step folds its row into the episode's accumulators,
+// an episode's end writes the record.
+template <bool STORE_STATE = true, bool GEN = false, bool ACC = false>
 __device__ __forceinline__ StepThreadOut step_env(const GteParams& P, const GteData& D, const GteState& S,
                                                   const StepConsts& K, const GteStepOut& O, uint64_t tick, int ring_slot,
                                                   int autoreset, int i, const EnvIn& in, const double p0, const double p1,
@@ -199,16 +250,21 @@ __device__ __forceinline__ StepThreadOut step_env(const GteParams& P, const GteD
         const DynRow row = {dyn_rp, dyn_pr, dyn_rew, dyn_prog, e.pos_idx};
         ring_store<GEN>(P, K.dyn, S, i, ring_slot, row);
     }
+    EpisodeAcc ea;
+    if (ACC) ea = episode_acc_fold(P, S, i, pos_tab[in.e.pos_idx], pos_tab[e.pos_idx], val, rew);
     acc.sum_rew = dadd(acc.sum_rew, rew);
     if (done || trunc) {                                                     // :269-271 calculate_metrics
         acc.episodes += 1;
         acc.terminated += done ? 1 : 0;
         acc.truncated += trunc ? 1 : 0;
         acc.sum_len += e.step;
-        acc.sum_pr = dadd(acc.sum_pr, dsub(ddiv(val, P.v0), 1.0));           // :282
-        acc.sum_mr = dadd(acc.sum_mr, dsub(ddiv(p1, __ldg(price + e.ep_start)), 1.0));   // :281
+        const double pr = dsub(ddiv(val, P.v0), 1.0);                        // :282
+        const double mr = dsub(ddiv(p1, __ldg(price + e.ep_start)), 1.0);    // :281
+        acc.sum_pr = dadd(acc.sum_pr, pr);
+        acc.sum_mr = dadd(acc.sum_mr, mr);
+        if (ACC) episode_record(P, O, i, ea, mr, pr, e.step);               // terminal values, before the auto-reset
         if (autoreset) {
-            reset_env<GEN>(P, D, S, i, tick, ring_slot, e, K.dyn);           // in-place auto-reset
+            reset_env<GEN, ACC>(P, D, S, i, tick, ring_slot, e, K.dyn);      // in-place auto-reset
             idx = e.ep_start;
             dyn_pos = dyn_rp = (float)pos_tab[e.pos_idx];                // first row: (position, position) :191-192
             dyn_pr = dyn_rew = dyn_prog = 0.0f;
@@ -224,8 +280,8 @@ __device__ __forceinline__ StepThreadOut step_env(const GteParams& P, const GteD
     return r;
 }
 
-// load + transition of env i in one go (fused step+gather kernel)
-template <bool GEN = false>
+// load + transition of env i in one go (step kernel; fused step+gather kernel, which never runs with ACC)
+template <bool GEN = false, bool ACC = false>
 __device__ __forceinline__ StepThreadOut step_env_now(const GteParams& P, const GteData& D, const GteState& S,
                                                       const void* __restrict__ actions, const StepConsts& K,
                                                       const GteStepOut& O, uint64_t tick, int ring_slot, int autoreset,
@@ -233,7 +289,7 @@ __device__ __forceinline__ StepThreadOut step_env_now(const GteParams& P, const 
     const EnvIn in = load_env(P, D, S, actions, K, i);
     double p0, p1;
     load_prices(P, D, in, p0, p1);
-    return step_env<true, GEN>(P, D, S, K, O, tick, ring_slot, autoreset, i, in, p0, p1, acc, pos_tab);
+    return step_env<true, GEN, ACC>(P, D, S, K, O, tick, ring_slot, autoreset, i, in, p0, p1, acc, pos_tab);
 }
 
 // Dynamic column j of r: the value of the kind whose ring block column j reads.

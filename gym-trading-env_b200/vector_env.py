@@ -24,6 +24,9 @@ import torch
 from . import _cabi
 from .dynamic_features import (DeviceFeature, episode_progress_feature, parse_dynamic_features,  # noqa: F401
                                portfolio_return_feature, reward_feature)
+from . import episode_metrics as _em
+from .episode_metrics import (DeviceMetric, episode_length_metric, episode_reward_metric,  # noqa: F401
+                              max_drawdown_metric, position_changes_metric, time_in_market_metric)
 from .data import SeriesArrays, build_window_tables, frame_to_arrays, load_frame, reconcile_series
 
 
@@ -402,6 +405,8 @@ class TradingVectorEnv(_VectorEnvBase):
         self._tick = 0
         self._needs_first = True
         self.log_metrics = []
+        self._episode_acc = None             # add_metric(): f64 [5, N] running state of each env's episode, or None
+        self._episode_record = None          # add_metric(): f64 [7, N] metrics of each env's last finished episode
 
         series = df if isinstance(df, (list, tuple)) else [df]
         series = [s if isinstance(s, SeriesArrays) else frame_to_arrays(s) for s in series]
@@ -1334,6 +1339,57 @@ class TradingVectorEnv(_VectorEnvBase):
         return torch.where(self._info_t["step"] > 0, act, state)
 
     # ------------------------------------------------------------------ metrics / errors / state
+    def add_metric(self, name, function):
+        """``TradingEnv.add_metric(name, function)`` (environments.py:274-276): record ``function`` over every env's
+        episode.  ``function`` must be a :class:`DeviceMetric` from the device catalogue (``episode_metrics.py``:
+        position_changes, episode_length, max_drawdown, episode_reward, time_in_market), accumulated in the step kernel
+        and recorded bit for bit at each episode's end; anything else raises NotImplementedError.  Call it before the
+        first ``reset()``, as the reference's usage does: the accumulators must run from an episode's reset row.  A
+        repeated name: the later function wins, as in the reference's metric dict."""
+        if not self._needs_first:
+            raise RuntimeError("add_metric() after reset(): episode metrics must be added before the first reset(), "
+                               "so that their accumulators run from every episode's reset row")
+        _em.check_metric_function(function)
+        self.log_metrics.append({"name": name, "function": function})
+        kinds = _em.metric_kinds_of(self.log_metrics)
+        N, f64 = self.num_envs, dict(dtype=torch.float64, device=self.device)
+        if self._episode_record is None:
+            self._episode_record = torch.full((_cabi.GTE_EPISODE_RECORD_ROWS, N), float("nan"), **f64)
+            self._O.episode_record = self._episode_record.data_ptr()
+        if kinds & _cabi.GTE_METRIC_KINDS_STATEFUL and self._episode_acc is None:
+            self._episode_acc = torch.zeros(_cabi.GTE_EPISODE_ACC_ROWS, N, **f64)
+            self._S.episode_acc = self._episode_acc.data_ptr()
+        self._P.metric_kinds = kinds
+        self._graph = None                                   # kernel arguments changed: re-capture
+
+    def get_episode_metrics(self, env_index=None):
+        """The metrics of each env's most recently finished episode (``add_metric``).  ``env_index=None``: a dict
+        name -> f64 [N] CUDA tensor ("Market Return", "Portfolio Return" as fractions, then each added name), NaN
+        for an env that has not finished an episode yet; the tensors are views of a buffer that later steps overwrite.
+        ``env_index=i``: the reference's ``get_metrics()`` dict of env i (environments.py:285-294) — the two returns
+        as its ``f"{100*x:5.2f}%"`` strings, the added metrics as Python numbers; raises if env i has not finished an
+        episode.  The record is kept across ``reset()``, as the reference keeps ``results_metrics``."""
+        if self._episode_record is None:
+            raise RuntimeError("no episode metric is configured: call add_metric(name, DeviceMetric) before reset()")
+        with torch.cuda.device(self.device):
+            self._lib.gte_serve_stop()                   # a resident server kernel owns the state while it runs
+        rows = _em.record_names(self.log_metrics)
+        if env_index is None:
+            return {name: self._episode_record[r] for name, r in rows.items()}
+        i = int(env_index)
+        if not 0 <= i < self.num_envs:
+            raise IndexError(f"env_index {env_index} out of range for {self.num_envs} envs")
+        rec = self._episode_record[:, i].cpu().numpy()
+        if np.isnan(rec[0]):
+            raise RuntimeError(f"env {i} has not finished an episode yet")
+        out = {}
+        for name, r in rows.items():
+            if r < 2:
+                out[name] = f"{100 * float(rec[r]):5.2f}%"
+            else:
+                out[name] = int(rec[r]) if _em.KINDS[r - 2] in _em.INT_KINDS else float(rec[r])
+        return out
+
     def get_metrics(self, total=True):
         """Numeric episode metrics (environments.py:279-283) as a name -> 0-d tensor dict."""
         t = self._metrics_total if total else self._metrics_step
@@ -1428,6 +1484,8 @@ class TradingVectorEnv(_VectorEnvBase):
         names = ["asset", "fiat", "interest_asset", "interest_fiat", "pos_idx", "step", "ep_start", "dataset_idx",
                  "dyn_ring", "ring_clock", "plan_cursor", "ds_used", "ds_episodes",
                  "metrics_total", "tick_dev"]
+        # episode metrics (add_metric): their accumulators and record, only when configured
+        names += [n for n in ("episode_acc", "episode_record") if getattr(self, "_" + n) is not None]
         return {n: getattr(self, "_" + n).clone() for n in names}
 
     def load_state_dict(self, d):
@@ -1453,7 +1511,7 @@ class TradingVectorEnv(_VectorEnvBase):
     @property
     def launches_per_step(self):
         """Kernel launches one `step()` of the on-device loop issues: 1 (windows=None, or transition + gather fused
-        into one launch for batches that fit a single wave), else 2 per env range."""
+        into one launch for batches that fit a single wave and no episode metric), else 2 per env range."""
         return int(self._lib.gte_step_obs_launches(C.byref(self._P), C.byref(self._D), self._obs_variant, self.n_chunks))
 
     @property

@@ -108,6 +108,36 @@ enum GteDynKind {
     GTE_DYN_EPISODE_PROGRESS = 5   /* history["step", -1] / max_episode_duration                                 */
 };
 
+/* Episode-metric kinds (GteParams.metric_kinds, bit 1 << kind): the device catalogue standing in for the reference's
+ * TradingEnv.add_metric(name, function) (environments.py:274-294).  Each value is computed in the step kernel in fp64,
+ * in the reference's operation order, over the episode's History (reset row included), and recorded at the episode's
+ * end in GteStepOut.episode_record row 2 + kind. */
+enum GteMetricKind {
+    GTE_METRIC_POSITION_CHANGES = 0, /* np.sum(np.diff(history["position"]) != 0): rows whose position differs from the previous row */
+    GTE_METRIC_EPISODE_LENGTH = 1,   /* len(history["position"]) = terminal step + 1                                               */
+    GTE_METRIC_MAX_DRAWDOWN = 2,     /* max(1 - v / running max(v)), v = history["portfolio_valuation"]                             */
+    GTE_METRIC_EPISODE_REWARD = 3,   /* sum(history["reward"]), Python's left-to-right sum                                          */
+    GTE_METRIC_TIME_IN_MARKET = 4    /* mean(history["position"] != 0)                                                              */
+};
+#define GTE_N_METRIC_KINDS 5
+#define GTE_METRIC_KINDS_ALL 0x1f
+/* Rows of GteState.episode_acc (f64 [GTE_EPISODE_ACC_ROWS, N]): the running state of the current episode.  Counts are
+ * stored as f64 (exact below 2^53).  Only the rows of configured kinds are read or written. */
+#define GTE_EPISODE_ACC_ROWS 5
+enum GteEpisodeAccRow {
+    GTE_ACC_PEAK = 0,                /* running max of the valuation (max_drawdown)                  */
+    GTE_ACC_DRAWDOWN = 1,            /* max drawdown so far (max_drawdown)                           */
+    GTE_ACC_REWARD_SUM = 2,          /* sum of the rewards so far (episode_reward)                   */
+    GTE_ACC_POSITION_CHANGES = 3,    /* rows whose position differs from the previous row            */
+    GTE_ACC_IN_MARKET = 4            /* rows whose position is not 0 (time_in_market)                */
+};
+/* Rows of GteStepOut.episode_record (f64 [GTE_EPISODE_RECORD_ROWS, N]): row 0 the market return close[-1] / close[0] - 1,
+ * row 1 the portfolio return valuation[-1] / valuation[0] - 1 (environments.py:281-282), row 2 + k metric kind k. */
+#define GTE_EPISODE_RECORD_ROWS 7
+/* the kinds that keep per-episode state in episode_acc (episode_length is the terminal step + 1) */
+#define GTE_METRIC_KINDS_STATEFUL ((1 << GTE_METRIC_POSITION_CHANGES) | (1 << GTE_METRIC_MAX_DRAWDOWN) | \
+                                   (1 << GTE_METRIC_EPISODE_REWARD) | (1 << GTE_METRIC_TIME_IN_MARKET))
+
 enum GteErrorBit {
     GTE_E_ACTION_RANGE = 1, GTE_E_PAST_END = 2, GTE_E_PLAN_RANGE = 4, GTE_E_PLAN_EXHAUSTED = 8, GTE_E_NEGATIVE_ACTION = 16
 };
@@ -156,6 +186,10 @@ typedef struct GteParams {
     double reward_lo;                /*               reward_lo, reward_hi); defaults 1, -inf, +inf give   */
     double reward_hi;                /*               basic_reward_function bit for bit                    */
     double positions[GTE_MAX_POSITIONS]; /* `positions` (:98)                                          */
+    int32_t metric_kinds;            /* episode metrics (add_metric, :274-294): bit 1 << k for enum GteMetricKind k.  Non-zero
+                                        turns the per-episode record on (GteStepOut.episode_record, and GteState.episode_acc
+                                        for the kinds in GTE_METRIC_KINDS_STATEFUL); 0 = off, the record is not written */
+    int32_t pad_metric;              /* 0                                                              */
 } GteParams;
 
 /* Device-resident market data: what TradingEnv._set_df builds (environments.py:128-143). */
@@ -211,6 +245,9 @@ typedef struct GteState {
     uint64_t* tick;                  /* u64 [1]  event counter keying the Philox draws; every gte_reset /
                                         gte_step / gte_step_obs call advances it by one ON THE DEVICE, so
                                         a captured CUDA graph of a step replays with fresh draws       */
+    double* episode_acc;             /* f64 [GTE_EPISODE_ACC_ROWS, N] running state of the current episode (enum GteEpisodeAccRow),
+                                        initialised from the reset row by every reset and by the auto-reset; needed when
+                                        metric_kinds has a GTE_METRIC_KINDS_STATEFUL bit, else may be NULL            */
 } GteState;
 
 /* Outputs of one lockstep iteration.  reward / flags / valuation / real_position / info_* are the
@@ -247,6 +284,13 @@ typedef struct GteStepOut {
                                         then holds only the first ended_cap of them and the dense flags must be read)   */
     float* reward_f32;               /* f32 [N] or NULL: the reward ALSO rounded to float32 (numpy's cast) — the opt-in,
                                         LOSSY wire of a trainer that keeps float32 rewards anyway (stable-baselines3)   */
+    double* episode_record;          /* f64 [GTE_EPISODE_RECORD_ROWS, N], required when metric_kinds != 0 (read only then): the
+                                        metrics of each env's most recently FINISHED episode (row layout at
+                                        GTE_EPISODE_RECORD_ROWS; rows 2 + k only for configured kinds k).  Written at
+                                        an episode's end, from its terminal values, before the auto-reset; the columns of
+                                        the other envs are left untouched.  gte_rollout does not replicate it per
+                                        iteration: afterwards it holds the last episode each env finished.  With it, a
+                                        gte_step_obs call never takes the fused launch (gte_step_obs_launches says so) */
 } GteStepOut;
 
 /* Host side of one lockstep iteration for a HOST policy (gte_step_host): actions come from pinned host memory,
@@ -336,7 +380,8 @@ int gte_gather_obs(const GteParams* params, const GteData* data, const GteState*
 
 /* One whole lockstep iteration — what a vector env's step() returns: gte_step + gte_gather_obs.
  * n_chunks: 0 = the library's choice: ONE fused launch (every CTA advances its own envs, then gathers their windows)
- * while the batch fits a single wave with <= 256 envs per CTA (~100k envs on a B200), else two plain launches;
+ * while the batch fits a single wave with <= 256 envs per CTA (~100k envs on a B200) and metric_kinds == 0, else two
+ * plain launches;
  * 1 = always two plain launches (measured fastest for large batches, profiles/r01_tuning.md).  n_chunks > 1
  * is an opt-in experiment: the envs are cut into that many ranges and the step kernel of range c+1 runs beside the
  * gather of range c on a library-owned side stream (forked from and joined back into `stream` with events, so the
@@ -432,7 +477,8 @@ int gte_info(const GteParams* params, const GteData* data, const GteState* state
  * (bindings assert their own layout against it). */
 int gte_struct_size(int which);
 
-/* Kernel launches one gte_step_obs call issues for this shape: 1 (windows == 0, or the fused form), else 2 per env
+/* Kernel launches one gte_step_obs call issues for this shape: 1 (windows == 0, or the fused form, never taken with
+ * params->metric_kinds != 0), else 2 per env
  * range (host-only helper; asks the CUDA runtime for the gather kernel's occupancy, so it needs a device). */
 int gte_step_obs_launches(const GteParams* params, const GteData* data, int variant, int n_chunks);
 
