@@ -18,7 +18,7 @@ _LAZY = {"TradingVectorEnv", "MultiDatasetTradingVectorEnv", "basic_reward_funct
          "dynamic_feature_last_position_taken", "dynamic_feature_real_position", "shard_envs", "LazyInfos",
          "DeviceReward", "log_return_reward", "simple_return_reward"}
 _FEATURES = {"DeviceFeature", "parse_dynamic_features", "portfolio_return_feature", "reward_feature",
-             "episode_progress_feature"}
+             "episode_progress_feature", "current_drawdown_feature", "position_age_feature"}
 _METRICS = {"DeviceMetric", "position_changes_metric", "episode_length_metric", "max_drawdown_metric",
             "episode_reward_metric", "time_in_market_metric"}
 

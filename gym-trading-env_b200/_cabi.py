@@ -28,8 +28,10 @@ GTE_MAX_DYN = 5
 GTE_N_METRIC_KINDS = 5            # enum GteMetricKind: metric_kinds bit 1 << kind
 GTE_METRIC_KINDS_ALL = 0x1f
 GTE_METRIC_KINDS_STATEFUL = 0x1d  # every kind but episode_length keeps state in episode_acc
-GTE_EPISODE_ACC_ROWS = 5
+GTE_EPISODE_ACC_ROWS = 6
+GTE_ACC_POSITION_AGE = 5          # the episode_acc row read only with position_age: [5, N] suffices without it
 GTE_EPISODE_RECORD_ROWS = 7
+GTE_DYN_CURRENT_DRAWDOWN, GTE_DYN_POSITION_AGE = 6, 7   # enum GteDynKind: the stateful kinds (keep state in episode_acc)
 
 
 def ring_tile_bytes(windows: int, n_dyn: int, dyn_kinds: int) -> int:

@@ -24,8 +24,9 @@ int check_cuda(const char* fn, cudaError_t e) {
 
 #define GTE_REQUIRE(fn, cond) do { if (!(cond)) return fail_arg(fn, #cond); } while (0)
 
-// GteParams.n_dyn / dyn_kinds: 0 with the legacy n_dyn 0 or 2, else one kind code 1..5 per column, each at most once
-const char* bad_dyn_kinds(const GteParams* p) {
+// GteParams.n_dyn / dyn_kinds: 0 with the legacy n_dyn 0 or 2, else one kind code 1..7 per column, each at most once;
+// the stateful kinds (current_drawdown, position_age) keep their state in GteState.episode_acc
+const char* bad_dyn_kinds(const GteParams* p, const GteState* s) {
     if (p->n_dyn < 0 || p->n_dyn > GTE_MAX_DYN) return "dyn_kinds: n_dyn must be 0..GTE_MAX_DYN";
     const uint32_t k = (uint32_t)p->dyn_kinds;
     if (k == 0) return (p->n_dyn == 0 || p->n_dyn == 2) ? nullptr : "dyn_kinds: 0 (the defaults) needs n_dyn 0 or 2";
@@ -33,12 +34,14 @@ const char* bad_dyn_kinds(const GteParams* p) {
     unsigned seen = 0;
     for (int j = 0; j < p->n_dyn; ++j) {
         const uint32_t c = (k >> (4 * j)) & 15u;
-        if (c < GTE_DYN_POSITION || c > GTE_DYN_EPISODE_PROGRESS) return "dyn_kinds: kind code outside 1..5";
+        if (c < GTE_DYN_POSITION || c > GTE_DYN_POSITION_AGE) return "dyn_kinds: kind code outside 1..7";
         if (seen & (1u << c)) return "dyn_kinds: a kind appears twice";
         seen |= 1u << c;
     }
     if ((seen & (1u << GTE_DYN_EPISODE_PROGRESS)) && p->max_episode_duration <= 0)
         return "dyn_kinds: episode_progress needs max_episode_duration > 0";
+    if (gte::dyn_stateful(*p) && s->episode_acc == nullptr)
+        return "dyn_kinds: current_drawdown / position_age need episode_acc";
     return nullptr;
 }
 
@@ -55,7 +58,7 @@ int check_common(const char* fn, const GteParams* p, const GteData* d, const Gte
     GTE_REQUIRE(fn, p->n_envs > 0);
     GTE_REQUIRE(fn, p->n_positions > 0 && p->n_positions <= GTE_MAX_POSITIONS);
     GTE_REQUIRE(fn, p->windows >= 0);
-    if (const char* why = bad_dyn_kinds(p)) return fail_arg(fn, why);
+    if (const char* why = bad_dyn_kinds(p, s)) return fail_arg(fn, why);
     GTE_REQUIRE(fn, p->n_static >= 0 && p->n_static + p->n_dyn > 0);
     GTE_REQUIRE(fn, p->n_datasets >= 1 && p->n_datasets <= GTE_MAX_DATASETS);
     GTE_REQUIRE(fn, p->initial_position_idx >= -1 && p->initial_position_idx < p->n_positions);
@@ -282,7 +285,7 @@ int gte_struct_size(int which) {
 int gte_step_obs_launches(const GteParams* params, const GteData* data, int variant, int n_chunks) {
     if (params == nullptr || data == nullptr || n_chunks < 0 || n_chunks > 16) return GTE_ERR_ARG;
     if (params->windows == 0) return 1;
-    // (episode metrics: the fused form is never taken, step_obs_is_fused says so)
+    // (episode accumulators, gte::acc_on: the fused form is never taken, step_obs_is_fused says so)
     if (n_chunks == 0 && gte::default_chunks(params->n_envs) == 1 && gte::step_obs_is_fused(*params, *data, variant)) return 1;
     return 2 * (n_chunks == 0 ? gte::default_chunks(params->n_envs) : n_chunks);
 }

@@ -156,8 +156,8 @@ __device__ __forceinline__ int ring_slot_of(const GteParams& P, uint64_t clock) 
 // is known at compile time (RingLayout).
 constexpr uint32_t kDynPosBlock = 0xF, kDynNone = 0xE;
 struct DynLayout {
-    uint32_t col_src;     // nibble j: the ring block column j reads: f32 block 0..3, or kDynPosBlock (u8 position indices)
-    uint32_t kind_blk;    // nibble k (enum GteDynKind): the block of kind k, or kDynNone when it is not configured
+    uint32_t col_src;     // nibble j: the ring block column j reads: f32 block 0..4, or kDynPosBlock (u8 position indices)
+    uint32_t kind_blk;    // nibble k (enum GteDynKind 1..7): the block of kind k, or kDynNone when it is not configured
     int n_f32, n_pos;     // f32 blocks, position-index blocks (0 or 1)
     int tile_bytes;       // GTE_RING_TILE_BYTES_DYN(W, n_f32, n_pos)
     bool general;
@@ -203,7 +203,7 @@ static inline DynLayout dyn_layout(const GteParams& P) {
     L.kind_blk = 0u;
     for (int k = 0; k < 8; ++k) L.kind_blk |= kDynNone << (4 * k);
     int blk = 0;
-    for (int k = GTE_DYN_REAL_POSITION; k <= GTE_DYN_EPISODE_PROGRESS; ++k)     // f32 blocks in kind-code order
+    for (int k = GTE_DYN_REAL_POSITION; k <= GTE_DYN_POSITION_AGE; ++k)         // f32 blocks in kind-code order
         for (int j = 0; j < P.n_dyn; ++j)
             if (((kinds >> (4 * j)) & 15u) == (uint32_t)k) L.kind_blk = (L.kind_blk & ~(15u << (4 * k))) | ((uint32_t)blk++ << (4 * k));
     if (L.n_pos) L.kind_blk = (L.kind_blk & ~(15u << (4 * GTE_DYN_POSITION))) | (kDynPosBlock << (4 * GTE_DYN_POSITION));
@@ -218,19 +218,22 @@ static inline DynLayout dyn_layout(const GteParams& P) {
 // configured are ignored.
 struct DynRow {
     float rp, pr, rew, prog;      // real_position, portfolio_return, reward, episode_progress
+    float dd, age;                // current_drawdown, position_age (stateful: written by the ACC instantiations only)
     int pos_idx;                  // position: index into positions
 };
-// Writes row r of env i into ring slot `slot` (step and reset side); needs n_dyn > 0.
-template <bool GEN>
+// Writes row r of env i into ring slot `slot` (step and reset side); needs n_dyn > 0.  GEN && ACC: the stateful kinds
+// may be configured (they need the episode accumulators and are never the default pair; otherwise their stores are
+// not compiled).
+template <bool GEN, bool ACC = false>
 __device__ __forceinline__ void ring_store(const GteParams& P, const DynLayout& L, const GteState& S, int i, int slot,
                                            const DynRow& r) {
     const RingLayout<GEN> R{L};
     const int W = P.windows > 0 ? P.windows : 1;
     const int e = i & 31;
     uint8_t* tile = S.dyn_ring + (int64_t)(i >> 5) * R.tile_bytes(W);
-    const float v[4] = {r.rp, r.pr, r.rew, r.prog};
+    const float v[6] = {r.rp, r.pr, r.rew, r.prog, r.dd, r.age};
 #pragma unroll
-    for (int k = GTE_DYN_REAL_POSITION; k <= GTE_DYN_EPISODE_PROGRESS; ++k) {
+    for (int k = GTE_DYN_REAL_POSITION; k <= (GEN && ACC ? GTE_DYN_POSITION_AGE : GTE_DYN_EPISODE_PROGRESS); ++k) {
         const uint32_t b = R.kind_block(k);
         if (b < kDynNone) *reinterpret_cast<float*>(tile + GTE_RING_F32_OFFSET(W, (int)b, slot, e)) = v[k - GTE_DYN_REAL_POSITION];
     }
@@ -255,27 +258,32 @@ struct EnvRegs {          // the per-env state a step keeps in registers
     int pos_idx, step, ep_start, ds;
 };
 
-// Episode metrics (GteParams.metric_kinds, TradingEnv.add_metric :274-294): the running state of env i's episode in
-// GteState.episode_acc, one f64 row per quantity (enum GteEpisodeAccRow).  Only the rows of configured kinds are touched.
+// Episode metrics (GteParams.metric_kinds, TradingEnv.add_metric :274-294) and the stateful dynamic features: the
+// running state of env i's episode in GteState.episode_acc, one f64 row per quantity (enum GteEpisodeAccRow).  Only the
+// rows of configured kinds are touched; the peak row serves both max_drawdown and current_drawdown.
 __device__ __forceinline__ bool metric_on(const GteParams& P, int kind) { return (P.metric_kinds >> kind) & 1; }
+// the stateful dynamic feature of kind k is a column (compile-time false for GEN = false: never the default pair)
+template <bool GEN>
+__device__ __forceinline__ bool dyn_on(const RingLayout<GEN>& R, int k) { return R.kind_block(k) != kDynNone; }
 
 // The reset row (:186-197): valuation v0, reward 0, the episode's first position.
-__device__ __forceinline__ void episode_acc_init(const GteParams& P, const GteState& S, int i, double position) {
+template <bool GEN>
+__device__ __forceinline__ void episode_acc_init(const GteParams& P, const RingLayout<GEN>& R, const GteState& S, int i,
+                                                 double position) {
     const int64_t N = P.n_envs;
     double* __restrict__ A = S.episode_acc;
-    if (metric_on(P, GTE_METRIC_MAX_DRAWDOWN)) {
-        A[GTE_ACC_PEAK * N + i] = P.v0;
-        A[GTE_ACC_DRAWDOWN * N + i] = 0.0;                                    // 1 - v0 / v0
-    }
+    if (metric_on(P, GTE_METRIC_MAX_DRAWDOWN) || dyn_on(R, GTE_DYN_CURRENT_DRAWDOWN)) A[GTE_ACC_PEAK * N + i] = P.v0;
+    if (metric_on(P, GTE_METRIC_MAX_DRAWDOWN)) A[GTE_ACC_DRAWDOWN * N + i] = 0.0;        // 1 - v0 / v0
     if (metric_on(P, GTE_METRIC_EPISODE_REWARD)) A[GTE_ACC_REWARD_SUM * N + i] = 0.0;
     if (metric_on(P, GTE_METRIC_POSITION_CHANGES)) A[GTE_ACC_POSITION_CHANGES * N + i] = 0.0;
     if (metric_on(P, GTE_METRIC_TIME_IN_MARKET)) A[GTE_ACC_IN_MARKET * N + i] = (position != 0.0) ? 1.0 : 0.0;
+    if (dyn_on(R, GTE_DYN_POSITION_AGE)) A[GTE_ACC_POSITION_AGE * N + i] = 0.0;
 }
 
 // TradingEnv.reset (environments.py:163-199) preceded by MultiDatasetTradingEnv.reset (:393-400).
 // Rare path (once per episode): plan/rotation bookkeeping goes straight to global memory.
 // GEN: the general dynamic-feature catalogue (L.general), else no dynamic columns or the default pair (RingLayout).
-// ACC: episode metrics are configured (metric_kinds != 0): the episode's accumulators start from the reset row.
+// ACC: the episode accumulators run (an episode metric or a stateful dynamic feature): they start from the reset row.
 template <bool GEN = false, bool ACC = false>
 __device__ __forceinline__ void reset_env(const GteParams& P, const GteData& D, const GteState& S,
                                        int i, uint64_t tick, int ring_slot, EnvRegs& e, const DynLayout& L) {
@@ -328,10 +336,10 @@ __device__ __forceinline__ void reset_env(const GteParams& P, const GteData& D, 
     for (int k = 0; k < P.n_limit_positions; ++k)                            // self._limit_orders = {} (:168)
         S.limit_price[(int64_t)i * P.n_positions + S.limit_seq[k]] = __longlong_as_double(0x7ff8000000000000ll);
     if (P.n_dyn > 0) {                        // first obs row (:191-192): position, real_position = position, else 0
-        const DynRow r = {(float)position, 0.0f, 0.0f, 0.0f, e.pos_idx};
-        ring_store<GEN>(P, L, S, i, ring_slot, r);
+        const DynRow r = {(float)position, 0.0f, 0.0f, 0.0f, 0.0f, 0.0f, e.pos_idx};
+        ring_store<GEN, ACC>(P, L, S, i, ring_slot, r);
     }
-    if (ACC) episode_acc_init(P, S, i, position);
+    if (ACC) episode_acc_init(P, RingLayout<GEN>{L}, S, i, position);
 }
 
 }  // namespace gte

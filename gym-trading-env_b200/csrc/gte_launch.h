@@ -26,6 +26,19 @@ cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t sme
 int num_sms();
 int step_grid(int n_envs);
 
+// A stateful dynamic feature (current_drawdown, position_age) is among the first n_dyn columns of dyn_kinds.
+inline bool dyn_stateful(const GteParams& P) {
+    for (int j = 0; j < P.n_dyn && j < 8; ++j) {
+        const uint32_t c = ((uint32_t)P.dyn_kinds >> (4 * j)) & 15u;
+        if (c == GTE_DYN_CURRENT_DRAWDOWN || c == GTE_DYN_POSITION_AGE) return true;
+    }
+    return false;
+}
+// The episode accumulators (GteState.episode_acc) run: an episode metric or a stateful dynamic feature is configured.
+// Selects the ACC instantiations of the step, rollout, server and reset kernels, and rules out the fused step+gather
+// launch, which has none.
+inline bool acc_on(const GteParams& P) { return P.metric_kinds != 0 || dyn_stateful(P); }
+
 cudaError_t launch_step(const GteParams& P, const GteData& D, const GteState& S, const void* actions,
                         const GteStepOut& O, int autoreset, cudaStream_t stream);
 cudaError_t launch_step_range(const GteParams& P, const GteData& D, const GteState& S, const void* actions,

@@ -708,12 +708,12 @@ static cudaError_t plan_tma(const ObsShape& sh, int n_envs, bool fused, TmaPlan*
 }
 
 // Whether gte_step_obs runs this shape as ONE fused launch: the batch must be small enough for every CTA of the
-// single-wave grid to own at most kFusedMaxEnvs envs, and no episode metric may be configured (the fused kernel is not
-// instantiated with their accumulators: it sits at its register cap).  *plan is filled when it does.
+// single-wave grid to own at most kFusedMaxEnvs envs, and the episode accumulators must be off (acc_on: the fused kernel
+// is not instantiated with them, it sits at its register cap).  *plan is filled when it does.
 static cudaError_t fused_plan(const GteParams& P, const GteData& D, int variant, TmaPlan* plan, bool* eligible) {
     static const bool enabled = [] { const char* e = getenv("GTE_FUSED"); return e == nullptr || atoi(e) != 0; }();
     *eligible = false;
-    if (!enabled || P.windows <= 0 || P.metric_kinds != 0 || (variant != GTE_OBS_AUTO && variant != GTE_OBS_TMA) || !obs_tma_supported(P, D))
+    if (!enabled || P.windows <= 0 || acc_on(P) || (variant != GTE_OBS_AUTO && variant != GTE_OBS_TMA) || !obs_tma_supported(P, D))
         return cudaSuccess;
     const ObsShape sh = make_shape(P);
     if (tma_kernel(tma_config(sh), kTileEnvs, true, false, sh.dyn.general) == nullptr) return cudaSuccess;

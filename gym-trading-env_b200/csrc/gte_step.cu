@@ -18,8 +18,9 @@ namespace gte {
 // Each CTA owns `tiles_per_cta` CONSECUTIVE 256-env tiles: 1 while the grid fits on the GPU at once, more beyond that
 // (see step_tiles_per_cta).  GEN: the general dynamic-feature catalogue (K0.dyn); every kernel below that writes the
 // ring runs one code path, instantiated with GEN = false for no dynamic columns / the default pair, whose ring layout
-// is then known at compile time (RingLayout).  ACC (here and in every kernel below): episode metrics are configured
-// (metric_kinds != 0); the ACC = false instantiations are the kernels of a run without them.
+// is then known at compile time (RingLayout).  ACC (here and in every kernel below): the episode accumulators run
+// (acc_on: an episode metric or a stateful dynamic feature); the ACC = false instantiations are the kernels of a run
+// without them.
 template <int MIN_CTAS, bool GEN = false, bool ACC = false>
 __global__ void __launch_bounds__(kStepThreads, MIN_CTAS)
 step_kernel(const GteParams P, const GteData D, const GteState S, const void* __restrict__ actions, const StepConsts K0,
@@ -47,7 +48,7 @@ step_kernel(const GteParams P, const GteData D, const GteState S, const void* __
         if (valid) r = step_env_now<GEN, ACC>(P, D, S, actions, K, O, tick, ring_slot, autoreset, (int)i, acc, s_pos);
         // windows=None (environments.py:156-157): the observation is the single row idx, written by the step kernel
         // itself -> one launch per lockstep iteration at small N
-        if (obs_rows != nullptr) write_obs_rows<GEN>(P, D, K.dyn, obs_rows, i, valid, r, obs_on_host != 0);
+        if (obs_rows != nullptr) write_obs_rows<GEN, ACC>(P, D, K.dyn, obs_rows, i, valid, r, obs_on_host != 0);
     }
     reduce_metrics<kStepThreads>(acc, O, S, chunk_flags);
 }
@@ -99,7 +100,7 @@ rollout_kernel(const GteParams P, const GteData D, const GteState S, const void*
             const StepThreadOut r = step_env<false, GEN, ACC>(P, D, S, K, o, tick0 + (uint64_t)k, ring_slot_of(P, clock0 + 1ull + (uint64_t)k),
                                                          autoreset, (int)i, in, p0, p1, acc, s_pos, &e);
             if (obs_rows != nullptr && (keep_obs || k == n_steps - 1))
-                write_obs_rows<GEN>(P, D, K.dyn, obs_rows + (keep_obs ? (int64_t)k * N * F : 0), i, true, r, false);
+                write_obs_rows<GEN, ACC>(P, D, K.dyn, obs_rows + (keep_obs ? (int64_t)k * N * F : 0), i, true, r, false);
         }
     }
     if (valid) store_env(S, i, e);
@@ -211,7 +212,7 @@ serve_kernel(const GteParams P, const GteData D, const GteState S, const StepCon
             load_prices(P, D, in, p0, p1);
             r = step_env<true, GEN, ACC>(P, D, S, K, O, tick, ring_slot, autoreset, (int)i, in, p0, p1, acc, s_pos);
         }
-        if (obs_rows != nullptr) write_obs_rows<GEN>(P, D, K.dyn, obs_rows, i, valid, r, obs_on_host != 0);
+        if (obs_rows != nullptr) write_obs_rows<GEN, ACC>(P, D, K.dyn, obs_rows, i, valid, r, obs_on_host != 0);
         GteStepOut o = O;
         o.seq_value = seq;                               // what the last CTA publishes to the host when all is visible
         reduce_metrics<kStepThreads>(acc, o, S, kChunkFirst | kChunkLast);
@@ -378,7 +379,7 @@ cudaError_t launch_step_range(const GteParams& P, const GteData& D, const GteSta
     // ONE build: 3 CTAs per SM at 80 registers with no local-memory spills.  The 4-CTAs/SM build (64 registers, 18 STL /
     // 15 LDL) measures the same on the C5 shard (0.0925 vs 0.0930 ms): the kernel is bound by the issue rate of its
     // dependent fp64 chains, not by resident warps, loads or stores (profiles/r02_tuning.md has the diagnostic runs)
-    auto kern = P.metric_kinds != 0 ? (K.dyn.general ? step_kernel<3, true, true> : step_kernel<3, false, true>)
+    auto kern = acc_on(P) ? (K.dyn.general ? step_kernel<3, true, true> : step_kernel<3, false, true>)
                                     : (K.dyn.general ? step_kernel<3, true> : step_kernel<3>);
     return launch_pdl(kern, dim3(grid), dim3(kStepThreads), 0, stream, P, D, S, actions, K, O, autoreset, tpc,
                       env_begin, env_end, chunk_flags, obs_rows, obs_on_host ? 1 : 0);
@@ -393,7 +394,7 @@ cudaError_t launch_reset(const GteParams& P, const GteData& D, const GteState& S
                          int first, cudaStream_t stream) {
     const int grid = (P.n_envs + kStepThreads - 1) / kStepThreads;
     const DynLayout L = dyn_layout(P);
-    auto kern = P.metric_kinds != 0 ? (L.general ? reset_kernel<true, true> : reset_kernel<false, true>)
+    auto kern = acc_on(P) ? (L.general ? reset_kernel<true, true> : reset_kernel<false, true>)
                                     : (L.general ? reset_kernel<true> : reset_kernel<false>);
     kern<<<grid, kStepThreads, 0, stream>>>(P, D, S, mask, first, L);
     bump_tick_kernel<<<1, 1, 0, stream>>>(S.tick);
@@ -489,7 +490,7 @@ cudaError_t launch_rollout(const GteParams& P, const GteData& D, const GteState&
     if (rollout_is_persistent(P, n_steps, keep_obs)) {
         const int grid = (int)((N + kStepThreads - 1) / kStepThreads);
         const StepConsts K = make_step_consts(P);
-        auto kern = P.metric_kinds != 0 ? (K.dyn.general ? rollout_kernel<true, true> : rollout_kernel<false, true>)
+        auto kern = acc_on(P) ? (K.dyn.general ? rollout_kernel<true, true> : rollout_kernel<false, true>)
                                         : (K.dyn.general ? rollout_kernel<true> : rollout_kernel<false>);
         e = launch_pdl(kern, dim3(grid), dim3(kStepThreads), 0, stream,
                        P, D, S, actions, K, O, autoreset, n_steps, keep_obs, P.windows == 0 ? obs : (float*)nullptr);
@@ -702,7 +703,7 @@ cudaError_t launch_step_host(const GteParams& P, const GteData& D, const GteStat
             h->ctl->alive = 1u;
             const int grid = (int)((N + kStepThreads - 1) / kStepThreads);
             const StepConsts K = make_step_consts(p0);
-            auto kern = p0.metric_kinds != 0 ? (K.dyn.general ? serve_kernel<true, true> : serve_kernel<false, true>)
+            auto kern = acc_on(p0) ? (K.dyn.general ? serve_kernel<true, true> : serve_kernel<false, true>)
                                              : (K.dyn.general ? serve_kernel<true> : serve_kernel<false>);
             kern<<<grid, kStepThreads, 0, h->serve>>>(p0, D, S, K, o, autoreset, obs, io.obs_host != nullptr ? 1 : 0, h->ctl,
                                                       h->dctl, seq, serve_idle_ns());

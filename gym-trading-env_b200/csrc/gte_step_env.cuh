@@ -12,6 +12,7 @@ struct StepThreadOut {       // what the gather phase of the fused kernel needs 
     int idx, ep_start, ds;   // post-reset row index, episode start, dataset
     float dyn_pos, dyn_rp;   // the dynamic features of row idx (position, real_position), as written to the ring
     float dyn_pr, dyn_rew, dyn_prog;   // portfolio_return, reward, episode_progress of row idx (read when configured)
+    float dyn_dd, dyn_age;             // current_drawdown, position_age of row idx (ACC only, read when configured)
 };
 
 struct MetricAcc {           // per-thread accumulators (deterministic: fixed tile order per thread)
@@ -111,24 +112,28 @@ __device__ __forceinline__ void load_prices(const GteParams& P, const GteData& D
     p1 = __ldg(price + in.idx + 1);
 }
 
-// Episode metrics (ACC): the accumulators of env i after this step's History row (position after the market trade and
+// Episode accumulators (ACC): the state of env i after this step's History row (position after the market trade and
 // the limit orders, valuation, reward) has been folded in, in the reference's operation order.  Stored back every step.
+// current / age: the values of the stateful dynamic features for this row (0 when their kind is not configured).
 struct EpisodeAcc {
-    double peak, drawdown, reward_sum, changes, in_market;
+    double peak, drawdown, reward_sum, changes, in_market, current, age;
 };
-__device__ __forceinline__ EpisodeAcc episode_acc_fold(const GteParams& P, const GteState& S, int i, double pos_before,
-                                                       double pos_after, double val, double rew) {
+template <bool GEN>
+__device__ __forceinline__ EpisodeAcc episode_acc_fold(const GteParams& P, const RingLayout<GEN>& R, const GteState& S,
+                                                       int i, double pos_before, double pos_after, double val, double rew) {
     const int64_t N = P.n_envs;
     double* __restrict__ A = S.episode_acc;
-    EpisodeAcc a = {0.0, 0.0, 0.0, 0.0, 0.0};
-    if (metric_on(P, GTE_METRIC_MAX_DRAWDOWN)) {
+    EpisodeAcc a = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+    const bool dd_metric = metric_on(P, GTE_METRIC_MAX_DRAWDOWN);
+    if (dd_metric || dyn_on(R, GTE_DYN_CURRENT_DRAWDOWN)) {                  // one peak update for both consumers
         a.peak = __ldcg(A + GTE_ACC_PEAK * N + i);
-        a.drawdown = __ldcg(A + GTE_ACC_DRAWDOWN * N + i);
-        a.peak = (val > a.peak) ? val : a.peak;                              // np.maximum.accumulate(v)
+        if (dd_metric) a.drawdown = __ldcg(A + GTE_ACC_DRAWDOWN * N + i);
+        a.peak = (val > a.peak) ? val : a.peak;                              // np.maximum.accumulate(v) / np.max(v)
         const double d = dsub(1.0, ddiv(val, a.peak));                       // 1 - v / peak
-        a.drawdown = (d > a.drawdown) ? d : a.drawdown;                      // np.max
+        a.current = d;
+        if (dd_metric) a.drawdown = (d > a.drawdown) ? d : a.drawdown;       // np.max
         A[GTE_ACC_PEAK * N + i] = a.peak;
-        A[GTE_ACC_DRAWDOWN * N + i] = a.drawdown;
+        if (dd_metric) A[GTE_ACC_DRAWDOWN * N + i] = a.drawdown;
     }
     if (metric_on(P, GTE_METRIC_EPISODE_REWARD)) {                           // sum(): left to right
         a.reward_sum = dadd(__ldcg(A + GTE_ACC_REWARD_SUM * N + i), rew);
@@ -142,17 +147,24 @@ __device__ __forceinline__ EpisodeAcc episode_acc_fold(const GteParams& P, const
         a.in_market = __ldcg(A + GTE_ACC_IN_MARKET * N + i) + ((pos_after != 0.0) ? 1.0 : 0.0);
         A[GTE_ACC_IN_MARKET * N + i] = a.in_market;
     }
+    if (dyn_on(R, GTE_DYN_POSITION_AGE)) {                                   // rows since the position last changed
+        a.age = (pos_after != pos_before) ? 0.0 : __ldcg(A + GTE_ACC_POSITION_AGE * N + i) + 1.0;
+        A[GTE_ACC_POSITION_AGE * N + i] = a.age;
+    }
     return a;
 }
 
 // The episode of env i ended with this step: its metrics into GteStepOut.episode_record (rows: include/gte_b200.h).
+// Written only with metrics configured: with stateful dynamic features alone, episode_record may be NULL.
 __device__ __forceinline__ void episode_record(const GteParams& P, const GteStepOut& O, int i, const EpisodeAcc& a,
                                                double market_return, double portfolio_return, int step) {
     const int64_t N = P.n_envs;
     double* __restrict__ R = O.episode_record;
     const double len = (double)step + 1.0;                                   // len(history): the reset row + step rows
-    R[i] = market_return;
-    R[N + i] = portfolio_return;
+    if (P.metric_kinds != 0) {
+        R[i] = market_return;
+        R[N + i] = portfolio_return;
+    }
     if (metric_on(P, GTE_METRIC_POSITION_CHANGES)) R[(2 + GTE_METRIC_POSITION_CHANGES) * N + i] = a.changes;
     if (metric_on(P, GTE_METRIC_EPISODE_LENGTH)) R[(2 + GTE_METRIC_EPISODE_LENGTH) * N + i] = len;
     if (metric_on(P, GTE_METRIC_MAX_DRAWDOWN)) R[(2 + GTE_METRIC_MAX_DRAWDOWN) * N + i] = a.drawdown;
@@ -162,8 +174,9 @@ __device__ __forceinline__ void episode_record(const GteParams& P, const GteStep
 
 // The arithmetic of one transition.  STORE_STATE = false: the caller keeps the env's state in registers across iterations
 // (rollout / server kernels) and takes it back through e_out.  GEN: the general dynamic-feature catalogue (K.dyn).
-// ACC: episode metrics are configured (P.metric_kinds != 0): every step folds its row into the episode's accumulators,
-// an episode's end writes the record.
+// ACC: the episode accumulators run (acc_on: an episode metric or a stateful dynamic feature): every step folds its row
+// into them before the ring store, which takes the stateful features' values from them; with metrics, an episode's end
+// writes the record.
 template <bool STORE_STATE = true, bool GEN = false, bool ACC = false>
 __device__ __forceinline__ StepThreadOut step_env(const GteParams& P, const GteData& D, const GteState& S,
                                                   const StepConsts& K, const GteStepOut& O, uint64_t tick, int ring_slot,
@@ -240,18 +253,26 @@ __device__ __forceinline__ StepThreadOut step_env(const GteParams& P, const GteD
     }
     const RingLayout<GEN> R{K.dyn};
     float dyn_pos = (float)pos_tab[e.pos_idx], dyn_rp = (float)rp;        // fp64 -> fp32 as numpy casts (:154)
-    float dyn_pr = 0.0f, dyn_rew = (float)rew, dyn_prog = 0.0f;
+    float dyn_pr = 0.0f, dyn_rew = (float)rew, dyn_prog = 0.0f, dyn_dd = 0.0f, dyn_age = 0.0f;
     // each value only when its kind is configured (the transition is issue-bound on fp64 divides)
     if (R.kind_block(GTE_DYN_PORTFOLIO_RETURN) != kDynNone) dyn_pr = (float)dsub(ddiv(val, P.v0), 1.0);
     if (R.kind_block(GTE_DYN_EPISODE_PROGRESS) != kDynNone)
         dyn_prog = (float)ddiv((double)e.step, (double)P.max_episode_duration);
+    // the episode accumulators: folded before the ring store, which takes the stateful features' values from them.
+    // A stateful feature is never the default pair: GEN = false keeps the fold after the store, as the metrics-only
+    // kernels have always had it (the order is worth a register in their allocation)
+    EpisodeAcc ea;
+    if (ACC && GEN) {
+        ea = episode_acc_fold(P, R, S, i, pos_tab[in.e.pos_idx], pos_tab[e.pos_idx], val, rew);
+        dyn_dd = (float)ea.current;
+        dyn_age = (float)ea.age;
+    }
     // _get_obs write-back (:153-154); an auto-reset below overwrites the same slot with the new episode's first row
     if (P.n_dyn > 0) {
-        const DynRow row = {dyn_rp, dyn_pr, dyn_rew, dyn_prog, e.pos_idx};
-        ring_store<GEN>(P, K.dyn, S, i, ring_slot, row);
+        const DynRow row = {dyn_rp, dyn_pr, dyn_rew, dyn_prog, dyn_dd, dyn_age, e.pos_idx};
+        ring_store<GEN, ACC>(P, K.dyn, S, i, ring_slot, row);
     }
-    EpisodeAcc ea;
-    if (ACC) ea = episode_acc_fold(P, S, i, pos_tab[in.e.pos_idx], pos_tab[e.pos_idx], val, rew);
+    if (ACC && !GEN) ea = episode_acc_fold(P, R, S, i, pos_tab[in.e.pos_idx], pos_tab[e.pos_idx], val, rew);
     acc.sum_rew = dadd(acc.sum_rew, rew);
     if (done || trunc) {                                                     // :269-271 calculate_metrics
         acc.episodes += 1;
@@ -267,7 +288,7 @@ __device__ __forceinline__ StepThreadOut step_env(const GteParams& P, const GteD
             reset_env<GEN, ACC>(P, D, S, i, tick, ring_slot, e, K.dyn);      // in-place auto-reset
             idx = e.ep_start;
             dyn_pos = dyn_rp = (float)pos_tab[e.pos_idx];                // first row: (position, position) :191-192
-            dyn_pr = dyn_rew = dyn_prog = 0.0f;
+            dyn_pr = dyn_rew = dyn_prog = dyn_dd = dyn_age = 0.0f;
             if (P.n_datasets > 1) S.dataset_idx[i] = e.ds;
         }
     }
@@ -277,6 +298,7 @@ __device__ __forceinline__ StepThreadOut step_env(const GteParams& P, const GteD
     r.idx = idx; r.ep_start = e.ep_start; r.ds = e.ds;
     r.dyn_pos = dyn_pos; r.dyn_rp = dyn_rp;
     r.dyn_pr = dyn_pr; r.dyn_rew = dyn_rew; r.dyn_prog = dyn_prog;
+    r.dyn_dd = dyn_dd; r.dyn_age = dyn_age;
     return r;
 }
 
@@ -292,11 +314,14 @@ __device__ __forceinline__ StepThreadOut step_env_now(const GteParams& P, const 
     return step_env<true, GEN, ACC>(P, D, S, K, O, tick, ring_slot, autoreset, i, in, p0, p1, acc, pos_tab);
 }
 
-// Dynamic column j of r: the value of the kind whose ring block column j reads.
-template <bool GEN>
+// Dynamic column j of r: the value of the kind whose ring block column j reads.  GEN && ACC: the stateful kinds may be
+// configured.
+template <bool GEN, bool ACC = false>
 __device__ __forceinline__ float dyn_value(const RingLayout<GEN>& R, const StepThreadOut& r, int j) {
     if (R.is_pos(j)) return r.dyn_pos;
     const uint32_t b = (uint32_t)R.f32_block(j);
+    if (GEN && ACC && b == R.kind_block(GTE_DYN_CURRENT_DRAWDOWN)) return r.dyn_dd;
+    if (GEN && ACC && b == R.kind_block(GTE_DYN_POSITION_AGE)) return r.dyn_age;
     return b == R.kind_block(GTE_DYN_REAL_POSITION) ? r.dyn_rp : b == R.kind_block(GTE_DYN_PORTFOLIO_RETURN) ? r.dyn_pr
          : b == R.kind_block(GTE_DYN_REWARD) ? r.dyn_rew : r.dyn_prog;
 }
@@ -309,8 +334,8 @@ __device__ __forceinline__ float dyn_value(const RingLayout<GEN>& R, const StepT
 //                      fetching (row, dataset, dynamic features) of the owning env by shuffle -> full 128-byte stores.
 //                      For MAPPED HOST memory, where every partial-sector store is its own PCIe transaction
 //                      (4096 envs: 60 us -> 27 us per host step).
-// GEN: dynamic columns in P.dyn_kinds order (general catalogue), else the default pair (RingLayout).
-template <bool GEN = false>
+// GEN: dynamic columns in P.dyn_kinds order (general catalogue), else the default pair (RingLayout).  ACC: as dyn_value.
+template <bool GEN = false, bool ACC = false>
 __device__ __forceinline__ void write_obs_rows(const GteParams& P, const GteData& D, const DynLayout& L,
                                                float* __restrict__ obs_rows, int64_t i, bool valid, const StepThreadOut& r,
                                                bool coalesced) {
@@ -322,7 +347,7 @@ __device__ __forceinline__ void write_obs_rows(const GteParams& P, const GteData
             float* __restrict__ o = obs_rows + i * F;
             for (int c = 0; c < P.n_static; ++c) o[c] = __ldg(f + c);
             if (P.n_dyn > 0)
-                for (int j = 0; j < R.n_cols(); ++j) o[P.n_static + j] = dyn_value(R, r, j);
+                for (int j = 0; j < R.n_cols(); ++j) o[P.n_static + j] = dyn_value<GEN, ACC>(R, r, j);
         }
         return;
     }
@@ -338,9 +363,11 @@ __device__ __forceinline__ void write_obs_rows(const GteParams& P, const GteData
         q.dyn_pr = __shfl_sync(FULL, r.dyn_pr, e);
         q.dyn_rew = __shfl_sync(FULL, r.dyn_rew, e);
         q.dyn_prog = __shfl_sync(FULL, r.dyn_prog, e);
+        q.dyn_dd = (GEN && ACC) ? __shfl_sync(FULL, r.dyn_dd, e) : 0.0f;
+        q.dyn_age = (GEN && ACC) ? __shfl_sync(FULL, r.dyn_age, e) : 0.0f;
         const bool ok = __shfl_sync(FULL, (int)valid, e) != 0;
         if (ok) o[j] = c < P.n_static ? __ldg(D.features + ((int64_t)ds * P.t_stride + idx) * P.n_static + c)
-                                      : dyn_value(R, q, c - P.n_static);
+                                      : dyn_value<GEN, ACC>(R, q, c - P.n_static);
     }
 }
 

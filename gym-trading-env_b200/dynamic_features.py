@@ -11,6 +11,14 @@ each computed on the device in fp64 in the reference's operation order, bit for 
 - ``reward``: ``history["reward", -1]``, the step's reward (0 when terminated); reset row 0.0;
 - ``episode_progress``: ``history["step", -1] / D``, D = the env's int ``max_episode_duration``; reset row 0.0.
 
+Two STATEFUL kinds depend on the whole episode.  The step kernel keeps their running state per env in the episode
+accumulators it also keeps for ``add_metric`` (so they take the two-launch form of a windowed step, as metrics do):
+
+- ``current_drawdown``: ``1 - v[-1] / np.max(v)``, v = ``history["portfolio_valuation"]``; reset row 0.0;
+- ``position_age``: the number of History rows since the position last changed (by value, as the ``position_changes``
+  metric compares rows: -0.0 equals 0.0, and a limit order that undoes the step's trade is no change), counted back to
+  the reset row when it never changed; reset row 0.0.  A raw count, exact in float32 up to 2^24 rows.
+
 A :class:`DeviceFeature` is also callable on a reference ``History`` and returns exactly that expression: it is the
 executable specification of the device column (the env itself never calls it).
 """
@@ -18,9 +26,12 @@ from __future__ import annotations
 
 import numbers
 
+import numpy as np
+
 KINDS = ("position", "real_position", "portfolio_return", "reward", "episode_progress")
-KIND_CODES = {k: i + 1 for i, k in enumerate(KINDS)}       # enum GteDynKind (include/gte_b200.h)
-MAX_DYN = len(KINDS)                                        # GTE_MAX_DYN
+STATEFUL_KINDS = ("current_drawdown", "position_age")      # keep per-env state in the episode accumulators
+KIND_CODES = {k: i + 1 for i, k in enumerate(KINDS + STATEFUL_KINDS)}   # enum GteDynKind (include/gte_b200.h)
+MAX_DYN = len(KINDS)                                        # GTE_MAX_DYN: columns per env
 
 # the reference's two default functions (environments.py:20-24), passed back in by name
 _SENTINEL_KINDS = {"dynamic_feature_last_position_taken": "position", "dynamic_feature_real_position": "real_position"}
@@ -35,8 +46,8 @@ class DeviceFeature:
     ``max_episode_duration`` is required by, and only by, ``kind="episode_progress"``."""
 
     def __init__(self, kind, max_episode_duration=None):
-        if kind not in KINDS:
-            raise ValueError(f"kind must be one of {list(KINDS)}")
+        if kind not in KIND_CODES:
+            raise ValueError(f"kind must be one of {list(KIND_CODES)}")
         if kind == "episode_progress":
             if not _is_int(max_episode_duration) or max_episode_duration < 1:
                 raise ValueError(f"episode_progress needs an int max_episode_duration >= 1, got {max_episode_duration!r}")
@@ -56,6 +67,13 @@ class DeviceFeature:
             return history["portfolio_valuation", -1] / history["portfolio_valuation", 0] - 1
         if k == "reward":
             return history["reward", -1]
+        if k == "current_drawdown":
+            v = np.asarray(history["portfolio_valuation"], float)
+            return 1 - v[-1] / np.max(v)
+        if k == "position_age":
+            p = np.asarray(history["position"], float)
+            ch = np.flatnonzero(p[1:] != p[:-1])
+            return float(len(p) - 1 - (ch[-1] + 1 if len(ch) else 0))
         return history["step", -1] / self.max_episode_duration
 
     def __eq__(self, other):
@@ -87,6 +105,16 @@ def episode_progress_feature(max_episode_duration):
     return DeviceFeature("episode_progress", max_episode_duration)
 
 
+def current_drawdown_feature():
+    """``1 - valuation[-1] / max(valuation)``: how far the portfolio is below the episode's best valuation so far."""
+    return DeviceFeature("current_drawdown")
+
+
+def position_age_feature():
+    """History rows since the position last changed (0 on the row where it changed and on the reset row)."""
+    return DeviceFeature("position_age")
+
+
 def _kind_of(f):
     if isinstance(f, DeviceFeature):
         return f.kind
@@ -94,7 +122,8 @@ def _kind_of(f):
     if kind is None:
         raise NotImplementedError(
             "dynamic_feature_functions may only hold the device catalogue: DeviceFeature(kind) for kind in "
-            f"{list(KINDS)} (factories portfolio_return_feature(), reward_feature(), episode_progress_feature(D); "
+            f"{list(KINDS + STATEFUL_KINDS)} (factories portfolio_return_feature(), reward_feature(), "
+            "episode_progress_feature(D), current_drawdown_feature(), position_age_feature(); "
             "dynamic_feature_last_position_taken / dynamic_feature_real_position are 'position' / 'real_position'). "
             "Arbitrary Python callbacks over a History cannot run inside the CUDA step kernel and there is no CPU "
             f"fallback; got {f!r}")
@@ -108,7 +137,8 @@ def parse_dynamic_features(functions, max_episode_duration):
     int ``max_episode_duration``."""
     fns = list(functions)
     if len(fns) > MAX_DYN:
-        raise ValueError(f"at most {MAX_DYN} dynamic features (one per kind of {list(KINDS)}), got {len(fns)}")
+        raise ValueError(f"at most {MAX_DYN} dynamic features (each kind of {list(KIND_CODES)} at most once), "
+                         f"got {len(fns)}")
     kinds = [_kind_of(f) for f in fns]
     for k in set(kinds):
         if kinds.count(k) > 1:
@@ -122,3 +152,9 @@ def parse_dynamic_features(functions, max_episode_duration):
     for j, k in enumerate(kinds):
         code |= KIND_CODES[k] << (4 * j)
     return len(kinds), code
+
+
+def stateful_kinds_of(n_dyn, dyn_kinds):
+    """The stateful kinds among the n_dyn columns of a dyn_kinds code (parse_dynamic_features)."""
+    codes = {(dyn_kinds >> (4 * j)) & 15 for j in range(n_dyn)}
+    return [k for k in STATEFUL_KINDS if KIND_CODES[k] in codes]

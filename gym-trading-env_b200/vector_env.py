@@ -22,8 +22,9 @@ import numpy as np
 import torch
 
 from . import _cabi
-from .dynamic_features import (DeviceFeature, episode_progress_feature, parse_dynamic_features,  # noqa: F401
-                               portfolio_return_feature, reward_feature)
+from .dynamic_features import (DeviceFeature, current_drawdown_feature, episode_progress_feature,  # noqa: F401
+                               parse_dynamic_features, portfolio_return_feature, position_age_feature, reward_feature,
+                               stateful_kinds_of)
 from . import episode_metrics as _em
 from .episode_metrics import (DeviceMetric, episode_length_metric, episode_reward_metric,  # noqa: F401
                               max_drawdown_metric, position_changes_metric, time_in_market_metric)
@@ -301,8 +302,10 @@ class TradingVectorEnv(_VectorEnvBase):
     catalogue (log / simple return with scale and clip), and ``dynamic_feature_functions`` a list of up to five
     :class:`DeviceFeature` columns, each kind at most once, in any order (``position``, ``real_position`` — also
     spelled :func:`dynamic_feature_last_position_taken` / :func:`dynamic_feature_real_position` —
-    ``portfolio_return``, ``reward``, ``episode_progress``; see ``dynamic_features.py``): arbitrary Python callbacks
-    over a History cannot run inside the kernel and there is deliberately no CPU fallback (NotImplementedError).
+    ``portfolio_return``, ``reward``, ``episode_progress``, and the stateful ``current_drawdown`` and
+    ``position_age``, which keep per-env state in the episode accumulators; see ``dynamic_features.py``):
+    arbitrary Python callbacks over a History cannot run inside the kernel and there is deliberately no CPU fallback
+    (NotImplementedError).
 
     Returned tensors are persistent buffers overwritten by the next call: copy what you keep.
     """
@@ -405,7 +408,8 @@ class TradingVectorEnv(_VectorEnvBase):
         self._tick = 0
         self._needs_first = True
         self.log_metrics = []
-        self._episode_acc = None             # add_metric(): f64 [5, N] running state of each env's episode, or None
+        self._episode_acc = None             # f64 [5 or 6, N] running state of each env's episode (add_metric, stateful
+                                             # dynamic features), or None
         self._episode_record = None          # add_metric(): f64 [7, N] metrics of each env's last finished episode
 
         series = df if isinstance(df, (list, tuple)) else [df]
@@ -498,6 +502,12 @@ class TradingVectorEnv(_VectorEnvBase):
         # (unused without dynamic columns: then sized as for the default pair, the shape state_dict() has always had)
         tile = _cabi.ring_tile_bytes(W, self._n_dyn or 2, self._dyn_kinds)
         self._dyn_ring = torch.zeros((N + 31) // 32, tile, dtype=torch.uint8, device=dev)
+        # stateful dynamic features keep their running state in the episode accumulators: only the rows they touch
+        # (row GTE_ACC_POSITION_AGE only with position_age), so that a later add_metric() reuses the same buffer
+        stateful = stateful_kinds_of(self._n_dyn, self._dyn_kinds)
+        if stateful:
+            rows = _cabi.GTE_ACC_POSITION_AGE + ("position_age" in stateful)
+            self._episode_acc = f64(rows, N)
         self._ring_clock = torch.zeros(1, dtype=torch.int64, device=dev)
         self._error_flag = i32(1)
         self._tick_dev = torch.zeros(1, dtype=torch.int64, device=dev)
@@ -568,6 +578,7 @@ class TradingVectorEnv(_VectorEnvBase):
         s.reset_plan = None if self._reset_plan is None else self._reset_plan.data_ptr()
         s.error_flag = self._error_flag.data_ptr()
         s.tick = self._tick_dev.data_ptr()
+        s.episode_acc = None if self._episode_acc is None else self._episode_acc.data_ptr()
         o = _cabi.GteStepOut()
         o.reward, o.terminated, o.truncated = self._reward.data_ptr(), self._terminated.data_ptr(), self._truncated.data_ptr()
         o.valuation = self._valuation.data_ptr()
@@ -1357,7 +1368,8 @@ class TradingVectorEnv(_VectorEnvBase):
             self._episode_record = torch.full((_cabi.GTE_EPISODE_RECORD_ROWS, N), float("nan"), **f64)
             self._O.episode_record = self._episode_record.data_ptr()
         if kinds & _cabi.GTE_METRIC_KINDS_STATEFUL and self._episode_acc is None:
-            self._episode_acc = torch.zeros(_cabi.GTE_EPISODE_ACC_ROWS, N, **f64)
+            # rows 0..4: row GTE_ACC_POSITION_AGE is only read by the position_age dynamic feature
+            self._episode_acc = torch.zeros(_cabi.GTE_ACC_POSITION_AGE, N, **f64)
             self._S.episode_acc = self._episode_acc.data_ptr()
         self._P.metric_kinds = kinds
         self._graph = None                                   # kernel arguments changed: re-capture
@@ -1484,7 +1496,7 @@ class TradingVectorEnv(_VectorEnvBase):
         names = ["asset", "fiat", "interest_asset", "interest_fiat", "pos_idx", "step", "ep_start", "dataset_idx",
                  "dyn_ring", "ring_clock", "plan_cursor", "ds_used", "ds_episodes",
                  "metrics_total", "tick_dev"]
-        # episode metrics (add_metric): their accumulators and record, only when configured
+        # episode metrics (add_metric) and stateful dynamic features: the accumulators and the record, only when configured
         names += [n for n in ("episode_acc", "episode_record") if getattr(self, "_" + n) is not None]
         return {n: getattr(self, "_" + n).clone() for n in names}
 
@@ -1511,7 +1523,8 @@ class TradingVectorEnv(_VectorEnvBase):
     @property
     def launches_per_step(self):
         """Kernel launches one `step()` of the on-device loop issues: 1 (windows=None, or transition + gather fused
-        into one launch for batches that fit a single wave and no episode metric), else 2 per env range."""
+        into one launch for batches that fit a single wave, no episode metric and no stateful dynamic feature), else 2
+        per env range."""
         return int(self._lib.gte_step_obs_launches(C.byref(self._P), C.byref(self._D), self._obs_variant, self.n_chunks))
 
     @property

@@ -99,13 +99,19 @@ enum GteRewardKind {
 
 /* Dynamic-feature kinds (GteParams.dyn_kinds): the device catalogue standing in for the reference's
  * `dynamic_feature_functions` (environments.py:43-48, :153-154).  Each column is the fp64 value cast to float32;
- * in an episode's first row (the reset row, :191-192) position and real_position read the position, the others 0. */
+ * in an episode's first row (the reset row, :191-192) position and real_position read the position, the others 0.
+ * The STATEFUL kinds (6, 7) depend on the whole episode: they keep their running state in GteState.episode_acc
+ * (row GTE_ACC_PEAK, shared with the max_drawdown metric, and row GTE_ACC_POSITION_AGE), so a configuration with
+ * one of them needs episode_acc.  Their f32 ring blocks follow the others in kind-code order. */
 enum GteDynKind {
     GTE_DYN_POSITION = 1,          /* history["position", -1]            (:20-21; u8 position index in the ring) */
     GTE_DYN_REAL_POSITION = 2,     /* history["real_position", -1]       (:23-24)                                */
     GTE_DYN_PORTFOLIO_RETURN = 3,  /* history["portfolio_valuation", -1] / history["portfolio_valuation", 0] - 1 */
     GTE_DYN_REWARD = 4,            /* history["reward", -1]: the step's reward (0 when terminated)               */
-    GTE_DYN_EPISODE_PROGRESS = 5   /* history["step", -1] / max_episode_duration                                 */
+    GTE_DYN_EPISODE_PROGRESS = 5,  /* history["step", -1] / max_episode_duration                                 */
+    GTE_DYN_CURRENT_DRAWDOWN = 6,  /* 1 - v[-1] / max(v), v = history["portfolio_valuation"] (stateful)          */
+    GTE_DYN_POSITION_AGE = 7       /* History rows since the position last changed (by value), back to the reset
+                                      row when it never did: a raw count, exact in f32 up to 2^24 (stateful)   */
 };
 
 /* Episode-metric kinds (GteParams.metric_kinds, bit 1 << kind): the device catalogue standing in for the reference's
@@ -122,14 +128,16 @@ enum GteMetricKind {
 #define GTE_N_METRIC_KINDS 5
 #define GTE_METRIC_KINDS_ALL 0x1f
 /* Rows of GteState.episode_acc (f64 [GTE_EPISODE_ACC_ROWS, N]): the running state of the current episode.  Counts are
- * stored as f64 (exact below 2^53).  Only the rows of configured kinds are read or written. */
-#define GTE_EPISODE_ACC_ROWS 5
+ * stored as f64 (exact below 2^53).  Only the rows of configured kinds are read or written: row 5 only when the
+ * position_age dynamic feature is configured, so a caller without that kind may allocate 5 rows ([5, N]). */
+#define GTE_EPISODE_ACC_ROWS 6
 enum GteEpisodeAccRow {
-    GTE_ACC_PEAK = 0,                /* running max of the valuation (max_drawdown)                  */
+    GTE_ACC_PEAK = 0,                /* running max of the valuation (max_drawdown, current_drawdown) */
     GTE_ACC_DRAWDOWN = 1,            /* max drawdown so far (max_drawdown)                           */
     GTE_ACC_REWARD_SUM = 2,          /* sum of the rewards so far (episode_reward)                   */
     GTE_ACC_POSITION_CHANGES = 3,    /* rows whose position differs from the previous row            */
-    GTE_ACC_IN_MARKET = 4            /* rows whose position is not 0 (time_in_market)                */
+    GTE_ACC_IN_MARKET = 4,           /* rows whose position is not 0 (time_in_market)                */
+    GTE_ACC_POSITION_AGE = 5         /* rows since the position last changed (position_age)          */
 };
 /* Rows of GteStepOut.episode_record (f64 [GTE_EPISODE_RECORD_ROWS, N]): row 0 the market return close[-1] / close[0] - 1,
  * row 1 the portfolio return valuation[-1] / valuation[0] - 1 (environments.py:281-282), row 2 + k metric kind k. */
@@ -174,7 +182,8 @@ typedef struct GteParams {
     int32_t dyn_kinds;               /* enum GteDynKind of dynamic column j in bits 4j..4j+3, each kind at most once.
                                         0 = the defaults: n_dyn == 0 none, n_dyn == 2 (position, real_position)
                                         (:20-24, :82), the same descriptor as the explicit 0x21.  episode_progress
-                                        needs max_episode_duration > 0                                           */
+                                        needs max_episode_duration > 0; current_drawdown and position_age need
+                                        GteState.episode_acc (rows 0..5 with position_age, else rows 0..4)       */
     int64_t t_stride;                /* rows allocated per dataset in `price` / `features`             */
     int64_t env_id_offset;           /* global index of env 0 (multi-GPU sharding; keys the RNG)       */
     uint64_t seed;                   /* Philox key                                                     */
@@ -247,7 +256,8 @@ typedef struct GteState {
                                         a captured CUDA graph of a step replays with fresh draws       */
     double* episode_acc;             /* f64 [GTE_EPISODE_ACC_ROWS, N] running state of the current episode (enum GteEpisodeAccRow),
                                         initialised from the reset row by every reset and by the auto-reset; needed when
-                                        metric_kinds has a GTE_METRIC_KINDS_STATEFUL bit, else may be NULL            */
+                                        metric_kinds has a GTE_METRIC_KINDS_STATEFUL bit or dyn_kinds a stateful kind
+                                        (6, 7), else may be NULL.  [5, N] suffices without position_age (row 5)     */
 } GteState;
 
 /* Outputs of one lockstep iteration.  reward / flags / valuation / real_position / info_* are the
@@ -380,8 +390,8 @@ int gte_gather_obs(const GteParams* params, const GteData* data, const GteState*
 
 /* One whole lockstep iteration — what a vector env's step() returns: gte_step + gte_gather_obs.
  * n_chunks: 0 = the library's choice: ONE fused launch (every CTA advances its own envs, then gathers their windows)
- * while the batch fits a single wave with <= 256 envs per CTA (~100k envs on a B200) and metric_kinds == 0, else two
- * plain launches;
+ * while the batch fits a single wave with <= 256 envs per CTA (~100k envs on a B200), metric_kinds == 0 and no stateful
+ * dynamic feature is configured, else two plain launches;
  * 1 = always two plain launches (measured fastest for large batches, profiles/r01_tuning.md).  n_chunks > 1
  * is an opt-in experiment: the envs are cut into that many ranges and the step kernel of range c+1 runs beside the
  * gather of range c on a library-owned side stream (forked from and joined back into `stream` with events, so the
@@ -478,7 +488,7 @@ int gte_info(const GteParams* params, const GteData* data, const GteState* state
 int gte_struct_size(int which);
 
 /* Kernel launches one gte_step_obs call issues for this shape: 1 (windows == 0, or the fused form, never taken with
- * params->metric_kinds != 0), else 2 per env
+ * params->metric_kinds != 0 or a stateful dynamic feature), else 2 per env
  * range (host-only helper; asks the CUDA runtime for the gather kernel's occupancy, so it needs a device). */
 int gte_step_obs_launches(const GteParams* params, const GteData* data, int variant, int n_chunks);
 
