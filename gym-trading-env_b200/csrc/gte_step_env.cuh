@@ -56,7 +56,8 @@ __device__ __forceinline__ void store_env(const GteState& S, int64_t i, const En
 struct EnvIn {
     EnvRegs e;
     int a;                // action: index into positions, or -1 = hold (out-of-range and negative actions included)
-    int idx, T;           // row before advancing (clamped to T-2 when the caller stepped past the data), dataset length
+    int idx, T;           // row before advancing (clamped to T-2, e.step with it, when the caller stepped past the data),
+                          // dataset length
 };
 
 // CG: load through L2 only — a kernel that stays resident across iterations (server kernel) must not find a line in
@@ -96,6 +97,9 @@ __device__ __forceinline__ EnvIn make_env_in(const GteParams& P, const GteData& 
     if (in.idx + 1 >= in.T) {        // stepping past the end of the data without a reset (caller bug)
         atomicOr(S.error_flag, GTE_E_PAST_END);
         in.idx = in.T - 2;
+        // the step counter moves back with the row: the transition stores row T-1 again, so every reader that starts
+        // from the stored state (gathers, info) stays inside the data
+        in.e.step = in.idx - in.e.ep_start;
     }
     return in;
 }

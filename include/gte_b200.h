@@ -146,6 +146,12 @@ enum GteEpisodeAccRow {
 #define GTE_METRIC_KINDS_STATEFUL ((1 << GTE_METRIC_POSITION_CHANGES) | (1 << GTE_METRIC_MAX_DRAWDOWN) | \
                                    (1 << GTE_METRIC_EPISODE_REWARD) | (1 << GTE_METRIC_TIME_IN_MARKET))
 
+/* GTE_E_PAST_END: an env stepped again after its episode reached the last row T-1 of its data (autoreset == 0, no reset
+ * in between).  The step is an ordinary transition from row T-2 to row T-1, computed from the env's current portfolio:
+ * the previous valuation is that portfolio valued at price[T-2] (portfolio_initial_value for an episode that started at
+ * T-2), the trade happens at price[T-2], then interest, then the valuation at price[T-1]; it is reported as truncated,
+ * counted in the batch metrics and folded into the episode accumulators like any truncation.  info idx / step and the
+ * stored row ep_start + step stay at T-1 (episode_progress does not grow), so no reader leaves the data. */
 enum GteErrorBit {
     GTE_E_ACTION_RANGE = 1, GTE_E_PAST_END = 2, GTE_E_PLAN_RANGE = 4, GTE_E_PLAN_EXHAUSTED = 8, GTE_E_NEGATIVE_ACTION = 16
 };
