@@ -179,8 +179,10 @@ class LazyInfos(Mapping):
 
     As in a SAME_STEP vector env the row describes the CURRENT state: for an env whose episode just ended it is the
     row `reset()` wrote for the new episode.  ``position_index`` is what the reference records: the action of the step
-    (hold -> -1, the reference's None) for envs that stepped, ``positions.index(position)`` for envs that were just
-    reset — read it before overwriting the action buffer passed to `step()`."""
+    (hold or out of range -> -1, the reference's None) for envs that stepped, ``positions.index(position)`` (the first
+    index holding an equal value) for envs that were just reset; after a masked `reset()` the envs outside the mask keep
+    their step row — read it before overwriting the action buffer passed to `step()`.  ``reward`` is the reward the
+    last `step()` returned, for every env (also where the row is a reset row, whose History reward is 0)."""
 
     BASE_KEYS = ["idx", "step", "position_index", "position", "real_position", "portfolio_valuation",
                  "dataset_idx", "portfolio_distribution_asset", "portfolio_distribution_fiat",
@@ -740,9 +742,14 @@ class TradingVectorEnv(_VectorEnvBase):
                 mask_ptr = C.c_void_p(keep.data_ptr())
             self._launch_reset(mask_ptr, first=False)
             self._launch_obs()
-            self._last_actions = None
+            if keep is None:
+                self._last_actions = None
+            elif self._last_actions is not None:
+                # the envs outside the mask keep their last step row; the reset envs read step == 0 (the reset row)
+                la = self._last_actions
+                self._last_actions = la.copy() if isinstance(la, np.ndarray) else la.clone()
             if self._track_ids is not None:
-                self._track_append(after_reset=True)
+                self._track_append(after_reset=True, mask=keep)
             return self._emit_obs(), self.infos
 
     def step(self, actions):
@@ -796,7 +803,9 @@ class TradingVectorEnv(_VectorEnvBase):
                     self._actions_dev.copy_(wide)
                     act, act_bytes = self._actions_dev, 8
             if self._track_ids is not None:
-                self._track_pre = (self._pos_idx[self._track_ids].clone(), self._dataset_idx[self._track_ids].clone())
+                # pre-step state of the tracked envs: the auto-reset overwrites the position and clears the limit orders
+                lim = None if self._limit_price is None else self._limit_price[self._track_ids].clone()
+                self._track_pre = (self._pos_idx[self._track_ids].clone(), self._dataset_idx[self._track_ids].clone(), lim)
             self._P.action_bytes = act_bytes
             self._last_actions = src if host_in else act
             try:
@@ -1224,35 +1233,61 @@ class TradingVectorEnv(_VectorEnvBase):
                    "portfolio_distribution_interest_asset", "portfolio_distribution_interest_fiat",
                    "reward", "terminated", "truncated", "dataset_idx", "new_episode",
                    # state after the in-place auto-reset (used to rebuild the reset() row of the next episode)
-                   "_post_idx", "_post_pos_idx", "_post_asset", "_post_fiat", "_post_ds"]
+                   "_post_idx", "_post_pos_idx", "_post_asset", "_post_fiat", "_post_ds",
+                   # 0 where a masked reset() left the env alone: no History row
+                   "_present"]
 
-    def _track_append(self, after_reset, actions=None):
+    def _first_position_index(self, pidx):
+        """``positions.index(positions[pidx])``: the FIRST index holding an equal value (environments.py:189) — what the
+        reference records in a reset row when ``positions`` lists a value twice (e.g. 0.0 and -0.0)."""
+        if getattr(self, "_pos_first", None) is None:
+            first = [self.positions.index(p) for p in self.positions]
+            self._pos_first = torch.tensor(first, dtype=torch.int32, device=self.device)
+        return self._pos_first[pidx.long()]
+
+    def _track_append(self, after_reset, actions=None, mask=None):
         if self._track_ids is None or self._track_len >= self._track_log.shape[0]:
             return
         i = self._track_ids
         z = torch.zeros(i.numel(), dtype=torch.float64, device=self.device)
         pos_tab = torch.tensor(self.positions, dtype=torch.float64, device=self.device)
+        dist = lambda a, f: [torch.where(a > 0, a, z), torch.where(f > 0, f, z),         # noqa: E731  max(0, x)
+                             torch.where(-a > 0, -a, z), torch.where(-f > 0, -f, z)]      # (portfolio.py:49-57)
         if after_reset:       # the row reset() writes (environments.py:186-197)
             pidx = self._pos_idx[i].long()
             pos = pos_tab[pidx]
             a, f = self._asset[i], self._fiat[i]
-            cols = [(self._ep_start[i] + self._step[i]).double(), self._step[i].double(), pidx.double(), pos, pos,
-                    torch.full_like(z, self.portfolio_initial_value), a.clamp(min=0), f.clamp(min=0),
-                    (-a).clamp(min=0), (-f).clamp(min=0), self._interest_asset[i], self._interest_fiat[i],
-                    z, z, z, self._dataset_idx[i].double(), z + 1, z, z, z, z, z]
+            present = z + 1 if mask is None else mask[i].double()
+            cols = [(self._ep_start[i] + self._step[i]).double(), self._step[i].double(),
+                    self._first_position_index(pidx).double(), pos, pos,
+                    torch.full_like(z, self.portfolio_initial_value), *dist(a, f),
+                    self._interest_asset[i], self._interest_fiat[i],
+                    z, z, z, self._dataset_idx[i].double(), z + 1, z, z, z, z, z, present]
         else:                 # the row step() adds (:253-264): terminal values where the episode ended
             pf = self._pre_reset_portfolio[:, i]
             a, f = pf[0], pf[1]
             a_i = actions[i]
-            pre_pos, pre_ds = self._track_pre
-            # position after the step (before any auto-reset) = target of the action unless it was a hold
-            pos = torch.where(a_i >= 0, pos_tab[a_i.clamp(min=0)], pos_tab[pre_pos.long()])
-            cols = [self._info_idx[i].double(), self._info_step[i].double(), a_i.double(), pos, self._real_position[i],
-                    self._valuation[i], a.clamp(min=0), f.clamp(min=0), (-a).clamp(min=0), (-f).clamp(min=0), pf[2], pf[3],
+            pre_pos, pre_ds, pre_lim = self._track_pre
+            # the position after the step, before any auto-reset, replayed from the pre-step state with the step
+            # kernel's comparisons (no arithmetic): an action outside [0, len(positions)) is a hold (:234)
+            valid = (a_i >= 0) & (a_i < len(self.positions))
+            target = torch.where(valid, a_i, torch.zeros_like(a_i))
+            cur = pre_pos.long()
+            cur = torch.where(valid & (pos_tab[target] != pos_tab[cur]), target, cur)          # :213-215
+            if pre_lim is not None and self._limit_seq_host:                                    # :217-223
+                row = self._info_idx[i].long()
+                hi, lo = self._high[pre_ds.long(), row], self._low[pre_ds.long(), row]
+                for pk in self._limit_seq_host:
+                    lim = pre_lim[:, pk]
+                    hit = (lim == lim) & (pos_tab[pk] != pos_tab[cur]) & (lim <= hi) & (lim >= lo)
+                    cur = torch.where(hit, torch.full_like(cur, pk), cur)
+            cols = [self._info_idx[i].double(), self._info_step[i].double(),
+                    torch.where(valid, a_i, torch.full_like(a_i, -1)).double(), pos_tab[cur], self._real_position[i],
+                    self._valuation[i], *dist(a, f), pf[2], pf[3],
                     self._reward[i], self._terminated[i].double(), self._truncated[i].double(),
                     pre_ds.double(), z,
                     (self._ep_start[i] + self._step[i]).double(), self._pos_idx[i].double(), self._asset[i], self._fiat[i],
-                    self._dataset_idx[i].double()]
+                    self._dataset_idx[i].double(), z + 1]
         self._track_log[self._track_len] = torch.stack(cols, dim=1)
         self._track_len += 1
 
@@ -1267,17 +1302,21 @@ class TradingVectorEnv(_VectorEnvBase):
         c = {n: k for k, n in enumerate(cols)}
         out = []
         for r in rows:
+            if not r[c["_present"]]:
+                continue
             out.append(r)
             if not r[c["new_episode"]] and (r[c["terminated"]] or r[c["truncated"]]) and self.autoreset:
                 # the row reset() writes for the episode the auto-reset started (environments.py:186-197)
                 n = np.zeros(len(cols))
-                pos = float(self.positions[int(r[c["_post_pos_idx"]])])
+                pos = self.positions[int(r[c["_post_pos_idx"]])]
                 a, f = r[c["_post_asset"]], r[c["_post_fiat"]]
-                n[c["idx"]], n[c["position_index"]], n[c["position"]], n[c["real_position"]] = r[c["_post_idx"]], r[c["_post_pos_idx"]], pos, pos
+                n[c["idx"]], n[c["position_index"]] = r[c["_post_idx"]], self.positions.index(pos)
+                n[c["position"]] = n[c["real_position"]] = float(pos)
                 n[c["portfolio_valuation"]] = self.portfolio_initial_value
-                n[c["portfolio_distribution_asset"]], n[c["portfolio_distribution_fiat"]] = max(a, 0.0), max(f, 0.0)
-                n[c["portfolio_distribution_borrowed_asset"]], n[c["portfolio_distribution_borrowed_fiat"]] = max(-a, 0.0), max(-f, 0.0)
-                n[c["dataset_idx"]], n[c["new_episode"]] = r[c["_post_ds"]], 1.0
+                # Python's max(0, x) (portfolio.py:49-57): the first argument wins a tie, so -0.0 reads +0.0
+                n[c["portfolio_distribution_asset"]], n[c["portfolio_distribution_fiat"]] = max(0.0, a), max(0.0, f)
+                n[c["portfolio_distribution_borrowed_asset"]], n[c["portfolio_distribution_borrowed_fiat"]] = max(0.0, -a), max(0.0, -f)
+                n[c["dataset_idx"]], n[c["new_episode"]], n[c["_present"]] = r[c["_post_ds"]], 1.0, 1.0
                 out.append(n)
         df = pd.DataFrame(np.array(out).reshape(-1, len(cols)), columns=cols)
         df = df[[n for n in cols if not n.startswith("_")]]
@@ -1338,6 +1377,8 @@ class TradingVectorEnv(_VectorEnvBase):
         """``position_index`` as the reference records it: the step's action (hold = None -> -1) for envs that stepped
         (:257), ``positions.index(position)`` on the row reset() writes (:189)."""
         state = self._info_t["position_index"]
+        if len(set(self.positions)) < len(self.positions):      # a value listed twice: the first index holding it
+            state = self._first_position_index(state)
         la = self._last_actions
         if la is None:
             return state

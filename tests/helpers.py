@@ -135,7 +135,12 @@ def assert_bits(a, b, what):
     a, b = np.ascontiguousarray(a), np.ascontiguousarray(b)
     assert a.shape == b.shape, f"{what}: shape {a.shape} vs {b.shape}"
     if a.tobytes() != b.astype(a.dtype).tobytes():
-        bad = np.argwhere(a != b.astype(a.dtype))
+        bb = b.astype(a.dtype)
+        bad = np.argwhere(a != bb)
+        if len(bad) == 0 and a.dtype.kind == "f":         # equal values, different bits: signed zeros or NaN payloads
+            bad = np.argwhere((np.signbit(a) != np.signbit(bb)) | (np.isnan(a) != np.isnan(bb)))
+        if len(bad) == 0:
+            raise AssertionError(f"{what}: the bytes differ")
         raise AssertionError(f"{what}: {len(bad)} elements differ bitwise, first at {bad[:3].tolist()}: "
                              f"{a[tuple(bad[0])]!r} vs {b[tuple(bad[0])]!r}")
 
